@@ -3,7 +3,7 @@
 encode) on synthetic graphs of the BASELINE.json shapes.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload powerlaw|reddit|wikipedia|flights]
+                    [--workload powerlaw|reddit|wikipedia|flights] [--dump-outputs DIR]
 
 Primary workload (all N): BASELINE.json configs[3], the one its metric ("... at 1/2/4/8 B200;
 % HBM roofline") is quoted on — a power-law temporal graph with 10M nodes, d=210, L=3, lazy
@@ -61,6 +61,8 @@ CHUNKED_NOTE = ('accumulation=chunked (opt-in, NOT the reference order): a row r
                 'order\'s own rounding error: against the exact (f64) result the sequential order is off by 2.4e-4, the '
                 'chunked one by 3e-6 (profiles/r02_accumulation_order_error.txt)')
 REF_DIR = os.path.join(ROOT, 'oracle', '_ref', 'TPNet')
+DUMP_BYTES = 64_000_000     # --dump-outputs: at most this much in all
+DUMP_STATE_ROWS = 2048
 
 
 def parse_args():
@@ -93,7 +95,17 @@ def parse_args():
     ap.add_argument('--pl-batch', type=int, default=PL_BATCH, help='power-law: edges per step and GPU')
     ap.add_argument('--scaling', default='weak', choices=['weak', 'strong'],
                     help='N > 1: weak = pl_batch edges per GPU and step (job batch pl_batch x N), strong = pl_batch in total')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='power-law, one GPU: after the timed steps, write what the last timed step computed as '
+                         'DIR/<name>.npy (float32 / float64), so that two builds can be compared output for output.  '
+                         'The other arms (the reddit / wikipedia / flights workloads, the sharded N > 1 path, '
+                         '--impl reference) write nothing and refuse the option')
+    args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs is not None and (args.impl != 'ours' or args.workload != 'powerlaw'):
+        ap.error('--dump-outputs applies to the power-law workload of --impl ours')
+    return args
 
 
 def peak_gbs():
@@ -600,7 +612,30 @@ def sharded_parity(args, rank, world, device):
     return out
 
 
-def run_powerlaw(args, rank, world, device, K, W, sampler, accumulation=None, with_e2e=True):
+def dump_outputs(out_dir, m, feats, step):
+    """What one step computed, as .npy files that two builds can be compared on: the decoder features of its calls
+    (`feats`: name -> [B, F], self.mlp included) and all L+1 layers of a sample of the rows its update wrote, decay
+    applied (get_random_projections).  Samples are drawn with fixed seeds from the step's own ids, so the same inputs
+    give the same files; the features are sampled too (with their row indices) only if they would not fit DUMP_BYTES."""
+    os.makedirs(out_dir, exist_ok=True)
+    touched = np.unique(np.concatenate([step[0], step[1]]))
+    ids = np.sort(np.random.default_rng(0).choice(touched, min(DUMP_STATE_ROWS, len(touched)), replace=False))
+    arrays = {'state_row_ids': ids.astype(np.float64),
+              'state_rows': torch.stack(m.get_random_projections(ids)).cpu().numpy()}     # [L+1, rows, d]
+    n = len(step[0])
+    row_bytes = sum(f.shape[1] for f in feats.values()) * 4
+    room = (DUMP_BYTES - 4096 - sum(a.nbytes for a in arrays.values())) // row_bytes
+    rows = None
+    if n > room:
+        rows = np.sort(np.random.default_rng(1).choice(n, room * row_bytes // (row_bytes + 8), replace=False))
+        arrays['feature_rows'] = rows.astype(np.float64)
+    for name, f in feats.items():
+        arrays[name + '_features'] = (f if rows is None else f[torch.from_numpy(rows).to(f.device)]).cpu().numpy()
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
+def run_powerlaw(args, rank, world, device, K, W, sampler, accumulation=None, with_e2e=True, dump=None):
     import torch.distributed as dist
     from tpnet_b200.sharded import ShardedRandomProjection
     accumulation = accumulation or args.accumulation
@@ -652,15 +687,17 @@ def run_powerlaw(args, rank, world, device, K, W, sampler, accumulation=None, wi
     nccl = world > 1 and not peer
     res = [(stage_nccl if nccl else stage)(st) for st in steps[warm_n:warm_n + K + W]]
 
-    def resident_pairs(st, which):
+    def resident_pairs(st, which, keep=None):
         with torch.no_grad():
             if world == 1:
-                m.get_pair_wise_feature(st['src'], st['dst' if which == 'pos' else 'neg'])
+                feat = m.get_pair_wise_feature(st['src'], st['dst' if which == 'pos' else 'neg'])[1]
             elif peer:
-                m.routed_pair_wise_feature(st['src'], st['dst' if which == 'pos' else 'neg'])
+                feat = m.routed_pair_wise_feature(st['src'], st['dst' if which == 'pos' else 'neg']).feat
             else:
                 _, feat = m.pair_wise_gram(None, None, plan=st[which])
-                m._head(feat)
+                feat = m._head(feat)
+        if keep is not None:
+            keep[which] = feat
 
     def resident_update(st):
         if nccl:
@@ -668,7 +705,7 @@ def run_powerlaw(args, rank, world, device, K, W, sampler, accumulation=None, wi
         else:
             m.update(st['src'], st['dst'], st['t'], next_time=st['t_last'])
 
-    def resident(st):
+    def resident(st, keep=None):
         if world == 1 and not args.no_prepare:
             # the half of the update that does not write the state starts now, on the module's side stream
             m.update_prepare(st['src'], st['dst'], st['t'], next_time=st['t_last'])
@@ -677,12 +714,12 @@ def run_powerlaw(args, rank, world, device, K, W, sampler, accumulation=None, wi
             cur, fs = torch.cuda.current_stream(device), m.feature_stream()
             fs.wait_stream(cur)
             with torch.cuda.stream(fs):
-                resident_pairs(st, 'neg')
-            resident_pairs(st, 'pos')
+                resident_pairs(st, 'neg', keep)
+            resident_pairs(st, 'pos', keep)
             cur.wait_stream(fs)
         else:
-            resident_pairs(st, 'pos')
-            resident_pairs(st, 'neg')
+            resident_pairs(st, 'pos', keep)
+            resident_pairs(st, 'neg', keep)
         resident_update(st)
 
     # Every step is captured once into a CUDA graph and replayed once, in order (the host-side launch latency of
@@ -698,13 +735,16 @@ def run_powerlaw(args, rank, world, device, K, W, sampler, accumulation=None, wi
             fn(*a)
         return gr
 
+    # --dump-outputs: the last timed step keeps its decoder features (in its graph's memory pool when captured)
+    last = {} if dump else None
+    keep = lambda i: last if i == len(res) - 1 else None     # noqa: E731
     if use_graphs:
         with torch.cuda.stream(side):
-            graphs = [capture(resident, st) for st in res]
+            graphs = [capture(resident, st, keep(i)) for i, st in enumerate(res)]
         torch.cuda.synchronize()
         run_step = lambda i: graphs[i].replay()              # noqa: E731
     else:
-        run_step = lambda i: resident(res[i])                # noqa: E731
+        run_step = lambda i: resident(res[i], keep(i))       # noqa: E731
     if world > 1:
         dist.barrier()
     for i in range(W):
@@ -725,7 +765,9 @@ def run_powerlaw(args, rank, world, device, K, W, sampler, accumulation=None, wi
     wall1 = time.perf_counter()
     dev_ms = sum(a.elapsed_time(b) for a, b in ev)
     m.check_errors()
-    del res
+    if dump:
+        dump_outputs(dump, m, last, steps[warm_n + K + W - 1])
+    del res, last
     if use_graphs:
         del graphs
 
@@ -974,7 +1016,7 @@ def main():
         if rank != 0:
             return
         if args.workload == 'powerlaw':
-            K = min(args.steps or 3, 6)
+            K = args.steps or 3
             W = min(args.warmup if args.warmup is not None else 1, 2)
             shape = powerlaw_shape(args)
             sec, n_small, kind = cpu_port_powerlaw(shape, args.pl_batch, W, K, threads, scale_down=10)
@@ -986,7 +1028,7 @@ def main():
                                f'batch {args.pl_batch}, CPU arm on a 10x down-scaled node set', 'batch': args.pl_batch}
         else:
             shape = SHAPES[args.workload]
-            K, W = min(args.steps or 30, 60), max(args.warmup or 3, 1)
+            K, W = args.steps or 30, max(args.warmup or 3, 1)
             warm_batches, steps = make_steps(shape, K + W, seed=0, warm=60)
             sec, kind = cpu_tpnet(shape, warm_batches, steps, W, K, threads)
             val = BATCH / sec
@@ -1005,6 +1047,8 @@ def main():
     # ---------------- our arm
     if not torch.cuda.is_available():
         raise SystemExit('bench.py (impl=ours) needs a CUDA device: there is no CPU fallback')
+    if args.dump_outputs is not None and world > 1:
+        raise SystemExit('--dump-outputs writes the outputs of a single-GPU run')
     import torch.distributed as dist
     torch.cuda.set_device(local_rank)
     device = torch.device('cuda', local_rank)
@@ -1017,7 +1061,7 @@ def main():
 
     if args.workload == 'powerlaw':
         K, W = args.steps or 20, max(args.warmup if args.warmup is not None else 3, 3)
-        line = run_powerlaw(args, rank, world, device, K, W, sampler)
+        line = run_powerlaw(args, rank, world, device, K, W, sampler, dump=args.dump_outputs)
         if world > 1 and not args.no_parity:
             parity = sharded_parity(args, rank, world, device)
             if rank == 0:

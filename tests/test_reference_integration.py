@@ -1,10 +1,11 @@
-"""Drop-in wiring against the real reference checkout (build container only: skipped when
-/root/reference is absent, e.g. on the GPU box).  No compute: the module has no CPU path; what is
+"""Drop-in wiring against the unmodified reference, as ``oracle/make_ref.py`` installs it into
+``oracle/_ref/TPNet`` (skipped where it is not installed).  No compute: the module has no CPU path; what is
 checked is that the reference's own loader accepts the synthetic datasets, that the launcher binds
 the CUDA-backed class under the reference's import, and that the reference assembles its model around it."""
 import dataclasses
 import logging
 import os
+import random
 import subprocess
 import sys
 
@@ -13,12 +14,13 @@ import pytest
 import torch
 
 import tpnet_b200
+from oracle.make_ref import ref_dir
 from tpnet_b200 import launch
 from tpnet_b200.synth import SHAPES, write_processed_dataset
 
-REF = '/root/reference'
-needs_reference = pytest.mark.skipif(not os.path.isfile(os.path.join(REF, 'models', 'TPNet.py')),
-                                     reason='reference checkout not present')
+REF = ref_dir()
+needs_reference = pytest.mark.skipif(not REF, reason='reference not installed (oracle/make_ref.py copies it from a '
+                                                     'TPNet checkout)')
 
 
 @pytest.fixture()
@@ -120,8 +122,27 @@ def test_launcher_gpu_sampler_option(in_tmp):
         'print(get_neighbor_sampler(data=None, sample_neighbor_strategy="uniform", seed=3), '
         'getattr(get_neighbor_sampler, "_tpn_gpu_sampler", False), sys.argv[1:])\n')
     repo = os.path.dirname(os.path.dirname(os.path.abspath(tpnet_b200.__file__)))
+    # --gpu 0: where CUDA is present the launcher selects that device, so it must exist on a one-GPU machine
     for extra, patched in (([], False), (['--tpn-gpu-sampler'], True)):
-        r = subprocess.run([sys.executable, '-m', 'tpnet_b200.launch', str(fake), 'probe.py', '--gpu', '1'] + extra,
+        r = subprocess.run([sys.executable, '-m', 'tpnet_b200.launch', str(fake), 'probe.py', '--gpu', '0'] + extra,
                            capture_output=True, text=True, cwd=repo, timeout=300)
         assert r.returncode == 0, r.stderr
-        assert r.stdout.strip().splitlines()[-1] == f"('reference sampler', 'uniform', 3) {patched} ['--gpu', '1']"
+        assert r.stdout.strip().splitlines()[-1] == f"('reference sampler', 'uniform', 3) {patched} ['--gpu', '0']"
+
+
+def test_launcher_selects_the_device_named_by_gpu(in_tmp, monkeypatch):
+    """`--gpu G` is parsed by the launcher and made the current CUDA device before the script runs (the reference
+    scripts only build the string 'cuda:G'); torch.cuda.set_device is recorded, so any G works on any machine."""
+    fake = in_tmp / 'checkout3'
+    (fake / 'models').mkdir(parents=True)
+    (fake / 'models' / 'TPNet.py').write_text('')
+    (fake / 'probe.py').write_text('import sys\nopen("argv.txt", "w").write(repr(sys.argv[1:]))\n')
+    chosen = []
+    monkeypatch.setattr(torch.cuda, 'is_available', lambda: True)
+    monkeypatch.setattr(torch.cuda, 'set_device', chosen.append)
+    monkeypatch.setattr(sys, 'argv', list(sys.argv))
+    monkeypatch.setattr(sys, 'path', list(sys.path))
+    monkeypatch.setattr(random, 'sample', random.sample)
+    launch.main([str(fake), 'probe.py', '--tpn-stock', '--gpu', '3'])       # --tpn-stock: nothing is imported or swapped
+    assert chosen == [3]
+    assert (fake / 'argv.txt').read_text() == repr(['--gpu', '3'])
