@@ -59,7 +59,7 @@
 extern "C" {
 #endif
 
-#define TPN_ABI_VERSION 11
+#define TPN_ABI_VERSION 12
 
 #define TPN_MAX_LAYERS 4
 
@@ -398,6 +398,12 @@ int tpn_route_update(const tpn_shard_t* sh, const int64_t* src_dev, const int64_
 int tpn_route_pairs(const tpn_shard_t* sh, const int64_t* a_dev, const int64_t* b_dev, int64_t n,
                     int64_t* a_rows_out, int64_t* b_rows_out, int64_t* keep_out, int32_t* count_out_dev,
                     void* ws_dev, size_t ws_bytes, void* stream);
+/* Global node ids -> rows of this rank's state: local row id / world if this rank owns the node, otherwise
+ * num_local_rows + a cache slot handed out through the mark table (reused if the node is already cached in this
+ * generation).  The slots handed out by this call are the ones the next tpn_pull_rows fills.  An id outside
+ * [0, global_nodes) sets counters[ERROR] = 1 and maps to row 0; a full cache sets ERROR = 2, as tpn_route_pairs does.
+ * Every id gets a row, in order (rows_out_dev holds n elements); n may be 0 (then the next pull fetches nothing). */
+int tpn_route_nodes(const tpn_shard_t* sh, const int64_t* ids_dev, int64_t n, int64_t* rows_out_dev, void* stream);
 /* Fills the cache slots handed out by the latest tpn_route_* call from the owners' memory (rows and, in lazy
  * mode, their stamps — a cached row is read exactly like a local one). */
 int tpn_pull_rows(const tpn_state_t* st, const tpn_shard_t* sh, void* stream);

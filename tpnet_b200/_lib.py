@@ -21,7 +21,7 @@ TPN_ERR_INDEX = -6
 STAGE_RAW, STAGE_ID_WRAP, STAGE_ID = 0, 1, 2
 TPN_MAX_LAYERS = 4
 UPDATE_WHOLE, UPDATE_PREPARE, UPDATE_APPLY = 0, 1, 2
-ABI_VERSION = 11
+ABI_VERSION = 12
 
 #: every symbol include/tpnet_b200.h declares (tests assert the .so exports all of them)
 EXPORTED_SYMBOLS = (
@@ -31,8 +31,9 @@ EXPORTED_SYMBOLS = (
     'tpn_stager_create', 'tpn_stager_destroy', 'tpn_stage',
     'tpn_update_messages', 'tpn_gather_blocks', 'tpn_set_debug_flags', 'tpn_pairwise_neighbors', 'tpn_head_forward',
     'tpn_planner_create', 'tpn_planner_destroy', 'tpn_plan', 'tpn_sampler_recent',
-    'tpn_route_workspace_bytes', 'tpn_route_update', 'tpn_route_pairs', 'tpn_pull_rows', 'tpn_peer_barrier',
-    'tpn_shard_new_generation', 'tpn_peer_alloc', 'tpn_peer_free', 'tpn_ipc_export', 'tpn_ipc_open', 'tpn_ipc_close',
+    'tpn_route_workspace_bytes', 'tpn_route_update', 'tpn_route_pairs', 'tpn_route_nodes', 'tpn_pull_rows',
+    'tpn_peer_barrier', 'tpn_shard_new_generation', 'tpn_peer_alloc', 'tpn_peer_free', 'tpn_ipc_export', 'tpn_ipc_open',
+    'tpn_ipc_close',
 )
 
 SHARD_CTR_NEED, SHARD_CTR_PREV, SHARD_CTR_ERROR, SHARD_COUNTERS = 0, 1, 2, 8
@@ -141,6 +142,8 @@ def _declare(lib: ctypes.CDLL) -> None:
     lib.tpn_route_pairs.restype = c_int
     lib.tpn_route_pairs.argtypes = [POINTER(TpnShard), c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p,
                                     c_void_p, c_void_p, c_size_t, c_void_p]
+    lib.tpn_route_nodes.restype = c_int
+    lib.tpn_route_nodes.argtypes = [POINTER(TpnShard), c_void_p, c_int64, c_void_p, c_void_p]
     lib.tpn_pull_rows.restype = c_int
     lib.tpn_pull_rows.argtypes = [POINTER(TpnState), POINTER(TpnShard), c_void_p]
     lib.tpn_peer_barrier.restype = c_int

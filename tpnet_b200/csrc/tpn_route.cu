@@ -9,6 +9,8 @@
 //             table indexed by global node id (int atomics; a slot number only decides where a row is cached,
 //             never a result) and stay valid until the next write to the state (one "generation"), so the
 //             update that follows the pair-wise calls of the same batch finds its rows already cached.
+//   nodes   : (tpn_route_nodes) a plain list of global ids, every one of them this rank's to read: each id gets a
+//             row — its local row if owned, else a cache slot handed out through the same mark table.  No compaction.
 //   pull    : one warp per new slot reads the row block of its node straight out of the owner's HBM over
 //             NVLink (peer pointers, IPC-mapped) and stores it in the extension row TOGETHER WITH THE OWNER'S
 //             STAMPS (lazy decay): a cached row is then read exactly like a local row — one multiply from its
@@ -88,6 +90,33 @@ __device__ __forceinline__ bool owned(const ShardView& sh, long long first, long
     return (int)(first % sh.world) == sh.rank;
 }
 
+// Remembers where the new extension slots of a routing call start (counters[PREV] = counters[NEED]): run by one
+// thread, in a launch that precedes every slot request of the call, so tpn_pull_rows fills exactly [PREV, NEED).
+__device__ __forceinline__ void mark_call_start(const ShardView& sh) {
+    const int need = sh.counters[TPN_SHARD_CTR_NEED];
+    sh.counters[TPN_SHARD_CTR_PREV] = need < sh.ext_rows ? need : (int)sh.ext_rows;
+}
+
+// Remote node s is read by this call: make sure it has a cache slot in this generation.  Only the first request of a
+// node claims one; the slot number is final once every request of the call has run (route_resolve_kernel, a later
+// launch, reads it from the mark).
+__device__ __forceinline__ void request_slot(const ShardView& sh, long long s) {
+    // a hub is the second endpoint of a large share of the batch (18 % on the power-law bench): test with a
+    // plain load first, so that only the requests that still see 0 — the first few — reach the atomic unit
+    // (measured, 800,000 pairs of the N=8 job: 47 us with the compare-and-swap alone).  The mark only moves
+    // 0 -> 1 -> slot + 2 within a generation, so a stale 0 just costs one failed compare-and-swap.
+    if (__ldcg(&sh.mark[s]) == 0 && atomicCAS(&sh.mark[s], 0, 1) == 0) {   // first request of this node in the generation
+        int slot = atomicAdd(&sh.counters[TPN_SHARD_CTR_NEED], 1);
+        if (slot >= sh.ext_rows) {                    // cache full: flagged, the access stays in bounds
+            sh.counters[TPN_SHARD_CTR_ERROR] = 2;
+            slot = 0;
+        } else {
+            sh.need_nodes[slot] = s;
+        }
+        atomicExch(&sh.mark[s], slot + 2);
+    }
+}
+
 __global__ void __launch_bounds__(kRouteThreads)
 route_count_kernel(ShardView sh, Items it, int* __restrict__ block_counts) {
     __shared__ int wsum[kRouteThreads / 32];
@@ -121,8 +150,7 @@ route_scan_kernel(ShardView sh, int* __restrict__ block_counts, int nblk, int* _
     __shared__ int carry_s;
     if (threadIdx.x == 0) {
         carry_s = 0;
-        const int need = sh.counters[TPN_SHARD_CTR_NEED];
-        sh.counters[TPN_SHARD_CTR_PREV] = need < sh.ext_rows ? need : (int)sh.ext_rows;
+        mark_call_start(sh);
     }
     __syncthreads();
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -187,20 +215,7 @@ route_scatter_kernel(ShardView sh, Items it, const int* __restrict__ block_offse
                 row = s / sh.world;
             } else {
                 row = -s - 1;
-                // a hub is the second endpoint of a large share of the batch (18 % on the power-law bench): test with a
-                // plain load first, so that only the requests that still see 0 — the first few — reach the atomic unit
-                // (measured, 800,000 pairs of the N=8 job: 47 us with the compare-and-swap alone).  The mark only moves
-                // 0 -> 1 -> slot + 2 within a generation, so a stale 0 just costs one failed compare-and-swap.
-                if (__ldcg(&sh.mark[s]) == 0 && atomicCAS(&sh.mark[s], 0, 1) == 0) {   // first request of this node in the generation
-                    int slot = atomicAdd(&sh.counters[TPN_SHARD_CTR_NEED], 1);
-                    if (slot >= sh.ext_rows) {                    // cache full: flagged, the access stays in bounds
-                        sh.counters[TPN_SHARD_CTR_ERROR] = 2;
-                        slot = 0;
-                    } else {
-                        sh.need_nodes[slot] = s;
-                    }
-                    atomicExch(&sh.mark[s], slot + 2);
-                }
+                request_slot(sh, s);
             }
             second_rows_out[pos] = row;
         }
@@ -209,14 +224,40 @@ route_scatter_kernel(ShardView sh, Items it, const int* __restrict__ block_offse
     }
 }
 
+// rows < 0 (-(global id) - 1) -> n_local + the node's slot.  count: device item count, or NULL when all `cap` are valid.
 __global__ void __launch_bounds__(256)
 route_resolve_kernel(ShardView sh, long long* __restrict__ second_rows, const int* __restrict__ count, long long cap) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    long long n = *count;
+    long long n = count != nullptr ? *count : cap;
     n = n < cap ? n : cap;
     if (i >= n) return;
     const long long v = second_rows[i];
     if (v < 0) second_rows[i] = sh.n_local + (long long)(sh.mark[-v - 1] - 2);
+}
+
+// tpn_route_nodes, first launch: the start of this call's slots (one thread).
+__global__ void __launch_bounds__(32) route_nodes_start_kernel(ShardView sh) {
+    if (threadIdx.x == 0) mark_call_start(sh);
+}
+
+// tpn_route_nodes, second launch: every id of the list -> local row, or -(id) - 1 with a slot requested.
+// An id outside the graph is flagged and maps to row 0.
+__global__ void __launch_bounds__(256)
+route_nodes_kernel(ShardView sh, const long long* __restrict__ ids, long long n, long long* __restrict__ rows_out) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const long long u = ids[i];
+    long long row;
+    if (u < 0 || u >= sh.global_nodes) {
+        sh.counters[TPN_SHARD_CTR_ERROR] = 1;
+        row = 0;
+    } else if ((int)(u % sh.world) == sh.rank) {
+        row = u / sh.world;
+    } else {
+        row = -u - 1;
+        request_slot(sh, u);
+    }
+    rows_out[i] = row;
 }
 
 // One warp per new extension slot: the owner's row block and stamps -> this rank's extension row.
@@ -374,6 +415,27 @@ extern "C" int tpn_route_pairs(const tpn_shard_t* sh, const int64_t* a_dev, cons
     it.n = n;
     return route_impl(sh, it, a_rows_out, b_rows_out, keep_out, nullptr, count_out_dev, ws_dev, ws_bytes,
                       reinterpret_cast<cudaStream_t>(stream_v));
+}
+
+extern "C" int tpn_route_nodes(const tpn_shard_t* sh, const int64_t* ids_dev, int64_t n, int64_t* rows_out_dev,
+                               void* stream_v) {
+    using namespace tpn;
+    int rc = validate_shard(sh);
+    if (rc != TPN_OK) return rc;
+    if (n < 0 || n > ((int64_t)1 << 34) || (n > 0 && (ids_dev == nullptr || rows_out_dev == nullptr)))
+        return TPN_ERR_INVALID_ARGUMENT;
+    DeviceScope scope(sh->mark);
+    cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_v);
+    const ShardView v = make_shard_view(sh);
+    // launched for an empty list too: the following tpn_pull_rows then has nothing to pull
+    route_nodes_start_kernel<<<1, 32, 0, stream>>>(v);
+    if (n > 0) {
+        const unsigned grid = (unsigned)((n + 255) / 256);
+        long long* rows = reinterpret_cast<long long*>(rows_out_dev);
+        route_nodes_kernel<<<grid, 256, 0, stream>>>(v, reinterpret_cast<const long long*>(ids_dev), n, rows);
+        route_resolve_kernel<<<grid, 256, 0, stream>>>(v, rows, nullptr, n);
+    }
+    return check_launch();
 }
 
 extern "C" int tpn_pull_rows(const tpn_state_t* st, const tpn_shard_t* sh, void* stream_v) {

@@ -15,6 +15,9 @@ no host plan and no collective —
   3. ``tpn_peer_barrier`` (flag words in peer memory) where the protocol needs one: after a write before the
      peers' next pull, and between the pulls of an update and its writes;
   4. the rank-local kernels with the device-side item count (``tpn_update_messages`` / ``tpn_pairwise``).
+The encoder's structured call and ``get_random_projections`` split their rows by position instead: every rank
+routes the ids its slice reads with ``tpn_route_nodes`` (own rows, or cache slots of the same mark table), pulls,
+and runs the plain kernels (``tpn_pairwise_neighbors`` / ``tpn_gather``) on the translated rows.
 All of it is plain kernel launches on one stream: a whole step can be captured in a CUDA graph.
 
 Data plane ``exchange='nccl'`` (portable; what the gloo CPU tests exercise): the routing plan is computed on
@@ -181,6 +184,8 @@ class ShardedRandomProjection(RandomProjectionModule):
     ``pair_wise_gram`` take the replicated global-id batch; ``pair_wise_gram`` returns the
     features of the pairs this rank owns together with their positions in the batch
     (``get_pair_wise_feature(..., gather=True)`` re-assembles the reference's ``[n, F]`` tensor on every rank).
+    ``neighbor_pair_wise_gram`` / ``get_neighbor_pair_wise_feature`` / ``get_random_projections`` compute a positional
+    slice of their rows on each rank and return it with its positions (``gather=True``: the reference's tensors).
 
     ``exchange``: 'peer' — routing, NVLink pulls and barriers on the device (module docstring; needs the state
     on CUDA); 'nccl' — host plan + one all_to_all_single; 'auto' — 'peer' when the state is created on a CUDA
@@ -535,6 +540,11 @@ class ShardedRandomProjection(RandomProjectionModule):
                 and arrays[0].shape[0] >= self.SLICED_UPLOAD_MIN
                 and all(a.shape[0] == arrays[0].shape[0] for a in arrays)):
             return self._sliced_upload(arrays, kinds)
+        return self._rank_ids_to_device(arrays, kinds)
+
+    def _rank_ids_to_device(self, arrays, kinds):
+        """Global ids of this rank's own lists (never the sliced upload of a replicated batch): host arrays are
+        range-checked against the global node count before anything is launched."""
         keep = self.node_num
         self.node_num = self.global_node_num          # the stager validates against node_num
         try:
@@ -748,6 +758,173 @@ class ShardedRandomProjection(RandomProjectionModule):
         pf[:feat.shape[0]] = feat
         pk[:feat.shape[0]] = keep
         return self.assemble(RoutedPairs(pk, pf, torch.tensor([feat.shape[0]], dtype=torch.int32, device=feat.device)), n)
+
+    # ------------------------------------------------------------------ node-list calls: encoder features, row reads
+    # A call with m rows (encoder rows, or ids of get_random_projections) is split by POSITION: rank r computes rows
+    # [r*per, min((r+1)*per, m)), per = ceil(m / world).  Every encoder row reads K + 2 node blocks wherever it runs, so
+    # no owner rule saves the pulls; the positional split balances the work exactly, and its size is known on the host
+    # (no device count, no capacity padding, no device -> host read).  The rows a rank reads are routed
+    # (tpn_route_nodes: own rows, or cache slots of the current generation) and pulled, then the plain kernels run on
+    # the translated rows of the local state.
+    def _row_split(self, m: int) -> Tuple[int, int, int]:
+        """(per, lo, hi): this rank computes rows [lo, hi) of a call with m rows."""
+        per = -(-m // self.world)
+        lo = min(self.rank * per, m)
+        return per, lo, min(lo + per, m)
+
+    def _positions(self, lo: int, hi: int) -> torch.Tensor:
+        """Device int64 [lo, hi) (cached: the same split recurs every batch)."""
+        key = ('positions', lo, hi)
+        t = self._route.get(key)
+        if t is None:
+            t = torch.arange(lo, hi, dtype=torch.int64, device=self._state.device)
+            if len(self._route) > 8:
+                self._route.clear()
+            self._route[key] = t
+        return t
+
+    def _check_node_call(self, what: str) -> None:
+        if self.world > 1 and self.exchange != 'peer':
+            raise NotImplementedError(f"{what} on a sharded state with world > 1 needs exchange='peer' "
+                                      f"(the 'nccl' data plane routes only update and the decoder pairs)")
+
+    def _route_node_rows(self, ids) -> torch.Tensor:
+        """Peer data plane: this rank's list of global ids (host array or CUDA tensor) -> int64 rows of the local state,
+        every remote row pulled into its cache slot.  Collective: every rank calls it (with its own list, possibly
+        empty), because the pull may take a barrier."""
+        lib = _lib.load()
+        n = int(len(ids))
+        rows = torch.empty(n, dtype=torch.int64, device=self._state.device)
+        ptr = self._rank_ids_to_device([ids], ['id'])[0] if n else None
+        rc = lib.tpn_route_nodes(self._c_shard(), ptr, n, rows.data_ptr() if n else None, self._stream())
+        if rc:
+            _lib.check(rc, 'tpn_route_nodes')
+        self._pull()
+        return rows
+
+    def _gather_slices(self, local: torch.Tensor, per: int, m: int) -> torch.Tensor:
+        """Every rank's slice of a positional split -> the [m, ...] tensor on every rank (one all_gather of the slices
+        padded to `per`; collective).  Not differentiable: the result is detached."""
+        if self.world == 1:
+            return local.detach()
+        if not dist.is_initialized():
+            raise RuntimeError('gather=True with world > 1 needs torch.distributed (one process per rank)')
+        rest = tuple(local.shape[1:])
+        if per == 0:
+            return local.detach()
+        pad = local.new_zeros((per,) + rest)
+        pad[:local.shape[0]] = local.detach()
+        full = local.new_empty((self.world * per,) + rest)
+        dist.all_gather_into_tensor(full, pad, group=self.group)
+        return full[:m]
+
+    def _nbr_gram_rows(self, lists, m: int, k: int) -> torch.Tensor:
+        """tpn_pairwise_neighbors on rows of the local state: lists = (nbr [m*K], src [m], dst [m]) as CUDA tensors or
+        already validated host arrays (staged here).  Node blocks too wide for the shared-memory staging take the plain
+        module's fallback, tpn_pairwise on the expanded row lists."""
+        dev = self._state.device
+        lib = _lib.load()
+        f = self.pair_wise_feature_dim
+        out = torch.empty(m, k, 2, f, dtype=torch.float32, device=dev)
+        if m == 0 or k == 0:
+            return out
+        ptrs = self._rank_ids_to_device(list(lists), ['id', 'id', 'id'])
+        st, stream, scale = self._c_state(), self._stream(), 0 if self.not_scale else 1
+        rc = lib.tpn_pairwise_neighbors(st, ptrs[0], ptrs[1], ptrs[2], m, k, scale, out.data_ptr(), stream)
+        if rc == _lib.TPN_ERR_UNSUPPORTED:
+            on_dev = [(a.to(dev) if isinstance(a, torch.Tensor) else
+                       torch.from_numpy(np.ascontiguousarray(a, dtype=np.int64)).to(dev)).contiguous() for a in lists]
+            tmp = torch.empty(m * k, f, dtype=torch.float32, device=dev)
+            for j, e in enumerate(on_dev[1:]):
+                e = e.repeat_interleave(k)
+                rc = lib.tpn_pairwise(st, on_dev[0].data_ptr(), e.data_ptr(), m * k, None, scale, tmp.data_ptr(), stream)
+                if rc:
+                    _lib.check(rc, 'tpn_pairwise')
+                out[:, :, j, :] = tmp.view(m, k, f)
+            self._h.launches += 2
+            return out
+        if rc:
+            _lib.check(rc, 'tpn_pairwise_neighbors')
+        self._h.launches += 1
+        return out
+
+    def neighbor_pair_wise_gram(self, neighbor_node_ids, src_node_ids, dst_node_ids):
+        """The encoder's structured call (TPNet.py:313-324) without the head, on the sharded state.  ``[m, K]`` global
+        neighbour ids and ``[m]`` src / dst ids, replicated on every rank; this rank computes the rows of its positional
+        slice.  Returns ``(positions in the batch, [rows, K, 2, F])``, the ``(keep, feat)`` convention of
+        ``pair_wise_gram``: block ``[j, k, 0]`` is the pair ``(nbr[keep[j], k], src[keep[j]])``, ``[j, k, 1]`` the pair
+        with ``dst``.  Peer data plane (or world 1); all ranks call it together."""
+        self._check_node_call('neighbor_pair_wise_gram')
+        dev = self._require_cuda()
+        if neighbor_node_ids.ndim != 2:
+            raise ValueError('neighbor_node_ids must be [m, num_neighbors]')
+        m, k = int(neighbor_node_ids.shape[0]), int(neighbor_node_ids.shape[1])
+        if len(src_node_ids) != m or len(dst_node_ids) != m:
+            raise ValueError('src and dst id arrays must have one entry per row of neighbor_node_ids')
+        per, lo, hi = self._row_split(m)
+        n = hi - lo
+        keep = self._positions(lo, hi)
+        resident = all(isinstance(a, torch.Tensor) and a.is_cuda for a in (neighbor_node_ids, src_node_ids, dst_node_ids))
+        if self.world == 1:
+            flat = neighbor_node_ids.reshape(-1)
+            return keep, self._nbr_gram_rows((flat, src_node_ids, dst_node_ids), m, k)
+        if resident:
+            ids = torch.cat([neighbor_node_ids[lo:hi].reshape(-1), src_node_ids[lo:hi], dst_node_ids[lo:hi]])
+        else:
+            host = [a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a)
+                    for a in (neighbor_node_ids, src_node_ids, dst_node_ids)]
+            ids = np.concatenate([host[0][lo:hi].reshape(-1), host[1][lo:hi], host[2][lo:hi]]).astype(np.int64,
+                                                                                                        copy=False)
+        rows = self._route_node_rows(ids)
+        nk = n * k
+        return keep, self._nbr_gram_rows((rows[:nk], rows[nk:nk + n], rows[nk + n:]), n, k)
+
+    def get_neighbor_pair_wise_feature(self, neighbor_node_ids, src_node_ids, dst_node_ids,
+                                       out: Optional[torch.Tensor] = None, gather: bool = False):
+        """TPNet.py:313-324 on the sharded state: ``self.mlp`` on the ``[rows*K*2, F]`` view of
+        ``neighbor_pair_wise_gram``.  Returns ``(positions in the batch, [rows, K, 2F])`` for this rank's slice (``out``:
+        the buffer for that slice); ``gather=True`` returns the reference's ``[m, K, 2F]`` on every rank (one
+        all_gather; collective).  The gathered tensor carries no gradient: training through a sharded state needs
+        the per-rank slices."""
+        keep, g = self.neighbor_pair_wise_gram(neighbor_node_ids, src_node_ids, dst_node_ids)
+        n, k = g.shape[0], g.shape[1]
+        f = self.pair_wise_feature_dim
+        flat_out = None if out is None else out.view(n * k * 2, f)
+        feat = self._head(g.view(n * k * 2, f), out=flat_out).view(n, k, 2 * f)
+        if not gather:
+            return keep, feat
+        m = int(neighbor_node_ids.shape[0])
+        return self._gather_slices(feat, self._row_split(m)[0], m)
+
+    def _gather_state_rows(self, ptr: int, n: int) -> torch.Tensor:
+        out = torch.empty(self.num_layer + 1, n, self.dim, dtype=torch.float32, device=self._state.device)
+        if n:
+            rc = _lib.load().tpn_gather(self._c_state(), ptr, n, out.data_ptr(), self._stream())
+            if rc:
+                _lib.check(rc, 'tpn_gather')
+            self._h.launches += 1
+        return out
+
+    def get_random_projections(self, node_ids, gather: bool = False):
+        """TPNet.py:101-110 on the sharded state: the L+1 rows of global ids, decay applied.  World 1 (the whole graph
+        is this rank's): the reference's list of L+1 ``[n, d]`` tensors, as on the plain module, ids checked against
+        the global node count.  World > 1 (peer data plane; all ranks call it together): this rank reads its positional
+        slice of ``node_ids`` and returns ``(positions, [L+1 tensors of shape rows x d])``; ``gather=True`` returns the
+        reference's list on every rank (one all_gather; collective, no gradient — the layers have none anyway)."""
+        self._check_node_call('get_random_projections')
+        dev = self._require_cuda()
+        n = int(len(node_ids))
+        if self.world == 1:
+            ptr = self._rank_ids_to_device([node_ids], ['id'])[0] if n else 0
+            out = self._gather_state_rows(ptr, n)
+            return [out[i] for i in range(self.num_layer + 1)]
+        per, lo, hi = self._row_split(n)
+        rows = self._route_node_rows(node_ids[lo:hi])
+        out = self._gather_state_rows(rows.data_ptr(), hi - lo)
+        if gather:
+            full = self._gather_slices(out.transpose(0, 1), per, n).transpose(0, 1).contiguous()
+            return [full[i] for i in range(self.num_layer + 1)]
+        return self._positions(lo, hi), [out[i] for i in range(self.num_layer + 1)]
 
     # ------------------------------------------------------------------ state changes invalidate the remote-row caches
     def _before_write(self) -> None:
