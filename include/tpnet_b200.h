@@ -59,7 +59,7 @@
 extern "C" {
 #endif
 
-#define TPN_ABI_VERSION 12
+#define TPN_ABI_VERSION 13
 
 #define TPN_MAX_LAYERS 4
 
@@ -331,6 +331,72 @@ int tpn_sampler_recent(const int64_t* offsets_dev, const int64_t* nbr_dev, const
                        const double* times_dev, int64_t num_nodes, const int64_t* q_nodes_dev,
                        const double* q_times_dev, int64_t n, int num_neighbors, int64_t* out_nbr_dev,
                        int64_t* out_eid_dev, double* out_times_dev, void* stream);
+
+/*
+ * Streaming `recent` sampler: the same answers as tpn_sampler_recent over every edge pushed so far, with the
+ * edges fed batch by batch in time order and no adjacency of the whole stream (SURVEY.md 8(d): the power-law
+ * stream is generated in batches and never materialised).  State is O(num_nodes * capacity) and lives on the device.
+ *
+ * Per node u two lists of at most `capacity` = C entries (neighbour, edge id, time), oldest first, row-major
+ * [num_nodes][C]:
+ *   ALL : the last C folded entries of u;
+ *   OLD : the last C folded entries of u strictly older than newest[u], the newest folded time of u (-inf: none).
+ * The latest pushed batch is PENDING: its 2B directed entries (per edge j: (dst, eid, t) for src, then (src, eid, t)
+ * for dst, utils/utils.py:248-251), stably sorted by node.  A push first FOLDS the previous pending batch into the
+ * lists, one warp per node with a pending segment and O(C + log B) work per node, then sorts the new batch.
+ *
+ * A query (u, t) returns the reference's row over all pushed edges when t >= newest[u] (the newest time of u before
+ * the latest push) — which TPNet's loop guarantees: it pushes a batch, queries at that batch's times, then pushes the
+ * next.  t > newest[u]: the last K of ALL ++ (pending entries of u older than t); t == newest[u]: the last K of OLD;
+ * t < newest[u]: not answerable exactly: the row is zero and err_flag gets TPN_STREAM_ERR_PAST.
+ *
+ * Device-side validation (bits OR-ed into *err_flag, which the caller polls; the offending item is dropped):
+ *   TPN_STREAM_ERR_INDEX : a pushed or queried node id outside [0, num_nodes)  (a dropped query gets a zero row)
+ *   TPN_STREAM_ERR_ORDER : a pushed time below the previous edge's time (or the previous batch's last time)
+ *   TPN_STREAM_ERR_PAST  : a query before newest[u]
+ * After a flagged push the answers are unspecified until tpn_stream_sampler_reset.
+ * Every table is allocated by the caller; tpn_stream_sampler_reset initialises them (it is the only call that
+ * touches every node).  push / query do no work proportional to num_nodes.
+ */
+#define TPN_STREAM_ERR_INDEX 1
+#define TPN_STREAM_ERR_ORDER 2
+#define TPN_STREAM_ERR_PAST 4
+typedef struct tpn_stream_sampler {
+    int64_t   num_nodes;
+    int32_t   capacity;     /* C >= 1: entries per list (the largest num_neighbors a query may ask for)      */
+    int32_t   reserved0;
+    int64_t   max_batch;    /* edges a push may carry: the pending arrays hold 2 * max_batch entries         */
+    int64_t*  all_nbr;      /* device [num_nodes][C]   ALL: neighbour ids                                     */
+    int64_t*  all_eid;      /* device [num_nodes][C]        edge ids                                          */
+    double*   all_t;        /* device [num_nodes][C]        times                                             */
+    int64_t*  old_nbr;      /* device [num_nodes][C]   OLD: neighbour ids                                     */
+    int64_t*  old_eid;      /* device [num_nodes][C]        edge ids                                          */
+    double*   old_t;        /* device [num_nodes][C]        times                                             */
+    int32_t*  all_cnt;      /* device [num_nodes]           entries in ALL                                    */
+    int32_t*  old_cnt;      /* device [num_nodes]           entries in OLD                                    */
+    double*   newest;       /* device [num_nodes]           newest folded time, -inf if none                  */
+    uint32_t* pend_node;    /* device [2 * max_batch]  pending entries sorted by node (num_nodes: dropped)    */
+    int64_t*  pend_nbr;     /* device [2 * max_batch]                                                         */
+    int64_t*  pend_eid;     /* device [2 * max_batch]                                                         */
+    double*   pend_t;       /* device [2 * max_batch]                                                         */
+    int32_t*  pend_count;   /* device int32[1]: pending entries (2B of the latest push)                       */
+    double*   last_time;    /* device double[1]: time of the last pushed edge, -inf if none                   */
+    int32_t*  err_flag;     /* device int32[1]: TPN_STREAM_ERR_* bits                                         */
+} tpn_stream_sampler_t;
+
+/* Scratch bytes tpn_stream_sampler_push needs for a batch of `batch` edges (the sort's buffers). */
+size_t tpn_stream_sampler_workspace_bytes(int64_t batch);
+/* All lists empty, newest = -inf, nothing pending, last_time = -inf, err_flag = 0. */
+int tpn_stream_sampler_reset(const tpn_stream_sampler_t* s, void* stream);
+/* Folds the pending batch, then makes (src_dev[j], dst_dev[j], eid_dev[j], t_dev[j]), j < batch <= max_batch, the
+ * pending batch.  Times must be non-decreasing and >= the previous batch's.  batch == 0 does nothing. */
+int tpn_stream_sampler_push(const tpn_stream_sampler_t* s, const int64_t* src_dev, const int64_t* dst_dev,
+                            const int64_t* eid_dev, const double* t_dev, int64_t batch, void* ws_dev, size_t ws_bytes,
+                            void* stream);
+/* tpn_sampler_recent's outputs for the edges pushed so far (num_neighbors <= capacity), under the condition above. */
+int tpn_stream_sampler_query(const tpn_stream_sampler_t* s, const int64_t* q_nodes_dev, const double* q_times_dev,
+                             int64_t n, int num_neighbors, int64_t* out_nbr_dev, int64_t* out_eid_dev,
+                             double* out_times_dev, void* stream);
 
 /*
  * Host-side routing plan of the node-sharded state (tpnet_b200/sharded.py; no reference counterpart —

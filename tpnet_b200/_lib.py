@@ -21,7 +21,7 @@ TPN_ERR_INDEX = -6
 STAGE_RAW, STAGE_ID_WRAP, STAGE_ID = 0, 1, 2
 TPN_MAX_LAYERS = 4
 UPDATE_WHOLE, UPDATE_PREPARE, UPDATE_APPLY = 0, 1, 2
-ABI_VERSION = 12
+ABI_VERSION = 13
 
 #: every symbol include/tpnet_b200.h declares (tests assert the .so exports all of them)
 EXPORTED_SYMBOLS = (
@@ -33,10 +33,12 @@ EXPORTED_SYMBOLS = (
     'tpn_planner_create', 'tpn_planner_destroy', 'tpn_plan', 'tpn_sampler_recent',
     'tpn_route_workspace_bytes', 'tpn_route_update', 'tpn_route_pairs', 'tpn_route_nodes', 'tpn_pull_rows',
     'tpn_peer_barrier', 'tpn_shard_new_generation', 'tpn_peer_alloc', 'tpn_peer_free', 'tpn_ipc_export', 'tpn_ipc_open',
-    'tpn_ipc_close',
+    'tpn_ipc_close', 'tpn_stream_sampler_workspace_bytes', 'tpn_stream_sampler_reset', 'tpn_stream_sampler_push',
+    'tpn_stream_sampler_query',
 )
 
 SHARD_CTR_NEED, SHARD_CTR_PREV, SHARD_CTR_ERROR, SHARD_COUNTERS = 0, 1, 2, 8
+STREAM_ERR_INDEX, STREAM_ERR_ORDER, STREAM_ERR_PAST = 1, 2, 4
 
 
 class TpnState(ctypes.Structure):
@@ -74,6 +76,32 @@ class TpnShard(ctypes.Structure):
         ('counters', c_void_p),
         ('need_nodes', c_void_p),
         ('barrier_seq', c_void_p),
+    ]
+
+
+class TpnStreamSampler(ctypes.Structure):
+    """Mirror of ``tpn_stream_sampler_t`` (include/tpnet_b200.h)."""
+    _fields_ = [
+        ('num_nodes', c_int64),
+        ('capacity', c_int32),
+        ('reserved0', c_int32),
+        ('max_batch', c_int64),
+        ('all_nbr', c_void_p),
+        ('all_eid', c_void_p),
+        ('all_t', c_void_p),
+        ('old_nbr', c_void_p),
+        ('old_eid', c_void_p),
+        ('old_t', c_void_p),
+        ('all_cnt', c_void_p),
+        ('old_cnt', c_void_p),
+        ('newest', c_void_p),
+        ('pend_node', c_void_p),
+        ('pend_nbr', c_void_p),
+        ('pend_eid', c_void_p),
+        ('pend_t', c_void_p),
+        ('pend_count', c_void_p),
+        ('last_time', c_void_p),
+        ('err_flag', c_void_p),
     ]
 
 
@@ -127,6 +155,16 @@ def _declare(lib: ctypes.CDLL) -> None:
     lib.tpn_sampler_recent.restype = c_int
     lib.tpn_sampler_recent.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int64,
                                        c_int, c_void_p, c_void_p, c_void_p, c_void_p]
+    lib.tpn_stream_sampler_workspace_bytes.restype = c_size_t
+    lib.tpn_stream_sampler_workspace_bytes.argtypes = [c_int64]
+    lib.tpn_stream_sampler_reset.restype = c_int
+    lib.tpn_stream_sampler_reset.argtypes = [POINTER(TpnStreamSampler), c_void_p]
+    lib.tpn_stream_sampler_push.restype = c_int
+    lib.tpn_stream_sampler_push.argtypes = [POINTER(TpnStreamSampler), c_void_p, c_void_p, c_void_p, c_void_p, c_int64,
+                                            c_void_p, c_size_t, c_void_p]
+    lib.tpn_stream_sampler_query.restype = c_int
+    lib.tpn_stream_sampler_query.argtypes = [POINTER(TpnStreamSampler), c_void_p, c_void_p, c_int64, c_int, c_void_p,
+                                             c_void_p, c_void_p, c_void_p]
     lib.tpn_planner_create.restype = c_int
     lib.tpn_planner_create.argtypes = [POINTER(c_void_p), c_int64, c_int, c_int]
     lib.tpn_planner_destroy.restype = None

@@ -8,10 +8,13 @@ ids, edge ids (int64) and times (float64), ``[n, num_neighbors]`` each.  The adj
 device as one CSR (built here once, per node stably sorted by timestamp); a query batch is one kernel
 (``tpn_sampler_recent``).  With ``as_tensors=True`` the results stay on the device and feed
 ``RandomProjectionModule.get_neighbor_pair_wise_feature`` without a host round trip.
+``StreamingRecentSampler`` gives the same answers without the whole edge list: it is fed batch by batch
+(``push``) and keeps O(num_nodes * max_neighbors) state on the device (``tpn_stream_sampler_*``).
 Only the `recent` strategy exists (what TPNet uses); there is no CPU path.
 """
 from __future__ import annotations
 
+import ctypes
 from typing import Tuple, Union
 
 import numpy as np
@@ -102,6 +105,176 @@ class RecentNeighborSampler:
         if as_tensors:
             return out_n, out_e, out_t
         return out_n.cpu().numpy(), out_e.cpu().numpy(), out_t.cpu().numpy()
+
+
+class StreamingRecentSampler:
+    """The `recent` sampler fed batch by batch: ``push(src, dst, edge_ids, t)`` appends one chronological batch,
+    and ``get_historical_neighbors`` answers exactly what ``RecentNeighborSampler`` built over every edge pushed so
+    far answers, for any query whose time is >= the node's newest time before the latest push.  TPNet's loop always
+    meets that condition: push the batch, query its src / dst / negatives at the batch's times, push the next.  A query
+    that breaks it cannot be answered exactly: it is flagged, and ``check_errors()`` raises.
+
+    No adjacency of the whole stream is built: the state is two lists of ``max_neighbors`` entries per node on the
+    device (48 * max_neighbors + 16 bytes per node) plus the latest batch (``tpn_stream_sampler_*``,
+    include/tpnet_b200.h), so streams that never exist as a whole edge list can be sampled.  ``push`` and
+    ``get_historical_neighbors`` with CUDA-tensor arguments never synchronise or allocate inside a CUDA-graph capture
+    (push batches of at most ``max_batch`` edges there; larger batches grow the buffers outside captures).
+    Host (numpy) arguments are validated before anything is launched; CUDA-tensor arguments are validated on the
+    device (the offending edge or query is dropped and flagged)."""
+
+    def __init__(self, num_nodes: int, max_neighbors: int, device: Union[str, torch.device], max_batch: int = 200_000):
+        dev = torch.device(device)
+        if dev.type != 'cuda':
+            raise RuntimeError('tpnet_b200.StreamingRecentSampler samples on CUDA only (no CPU fallback)')
+        if num_nodes < 1 or num_nodes > 0xffffffff:
+            raise ValueError('num_nodes must be in [1, 2**32)')
+        if max_neighbors < 1:
+            raise ValueError('max_neighbors must be positive')
+        if max_batch < 1:
+            raise ValueError('max_batch must be positive')
+        if dev.index is None:
+            dev = torch.device('cuda', torch.cuda.current_device())
+        self.device = dev
+        self.num_nodes = int(num_nodes)
+        self.max_neighbors = int(max_neighbors)
+        N, C = self.num_nodes, self.max_neighbors
+        i64, f64, i32 = torch.int64, torch.float64, torch.int32
+        self._lists = {k: torch.empty(N, C, dtype=d, device=dev) for k, d in
+                       (('all_nbr', i64), ('all_eid', i64), ('all_t', f64),
+                        ('old_nbr', i64), ('old_eid', i64), ('old_t', f64))}
+        self._all_cnt = torch.empty(N, dtype=i32, device=dev)
+        self._old_cnt = torch.empty(N, dtype=i32, device=dev)
+        self._newest = torch.empty(N, dtype=f64, device=dev)
+        self._pend_count = torch.zeros(1, dtype=i32, device=dev)
+        self._last_time = torch.empty(1, dtype=f64, device=dev)
+        self._err = torch.zeros(1, dtype=i32, device=dev)
+        self.max_batch = 0
+        self._ws = None
+        self._grow(int(max_batch))
+        self.sample_neighbor_strategy = 'recent'
+        self.seed = None
+        self.reset()
+
+    def _grow(self, max_batch: int) -> None:
+        """Pending arrays for 2 * max_batch entries (the current pending batch is kept) and the push workspace."""
+        if torch.cuda.is_current_stream_capturing():
+            raise RuntimeError(f'StreamingRecentSampler: a batch of {max_batch} edges exceeds max_batch='
+                               f'{self.max_batch} inside a CUDA-graph capture; construct it with a larger max_batch')
+        dev, cap = self.device, 2 * max_batch
+        pend = {'pend_node': torch.empty(cap, dtype=torch.int32, device=dev),     # uint32 keys in the C struct
+                'pend_nbr': torch.empty(cap, dtype=torch.int64, device=dev),
+                'pend_eid': torch.empty(cap, dtype=torch.int64, device=dev),
+                'pend_t': torch.empty(cap, dtype=torch.float64, device=dev)}
+        if self.max_batch:
+            for k, v in pend.items():
+                v[:2 * self.max_batch].copy_(self._pend[k])
+        self._pend = pend
+        need = int(_lib.load().tpn_stream_sampler_workspace_bytes(max_batch))
+        self._ws = torch.empty(need, dtype=torch.uint8, device=dev)
+        self.max_batch = max_batch
+        self._c = _lib.TpnStreamSampler(
+            num_nodes=self.num_nodes, capacity=self.max_neighbors, max_batch=max_batch,
+            **{k: v.data_ptr() for k, v in self._lists.items()}, **{k: v.data_ptr() for k, v in pend.items()},
+            all_cnt=self._all_cnt.data_ptr(), old_cnt=self._old_cnt.data_ptr(), newest=self._newest.data_ptr(),
+            pend_count=self._pend_count.data_ptr(), last_time=self._last_time.data_ptr(), err_flag=self._err.data_ptr())
+
+    def _stream(self) -> int:
+        return torch._C._cuda_getCurrentRawStream(self.device.index)
+
+    def _to_device(self, a: ArrayOrTensor, dtype: torch.dtype) -> torch.Tensor:
+        if isinstance(a, torch.Tensor):
+            return a.to(device=self.device, dtype=dtype).contiguous().reshape(-1)
+        return torch.from_numpy(np.ascontiguousarray(a, dtype=np.int64 if dtype == torch.int64 else np.float64)
+                                ).reshape(-1).to(self.device)
+
+    def reset_random_state(self) -> None:
+        """`recent` sampling is deterministic: nothing to reset (as RecentNeighborSampler)."""
+
+    def reset(self) -> None:
+        """Forget every pushed edge (a new epoch restarts the stream); clears the error flag."""
+        _lib.check(_lib.load().tpn_stream_sampler_reset(ctypes.byref(self._c), self._stream()),
+                   'tpn_stream_sampler_reset')
+        self._last_host = -np.inf           # last pushed time, when the host knows it (numpy pushes)
+
+    def push(self, src_node_ids: ArrayOrTensor, dst_node_ids: ArrayOrTensor, edge_ids: ArrayOrTensor,
+             node_interact_times: ArrayOrTensor) -> None:
+        """Appends one batch; its times are non-decreasing and >= every earlier pushed time."""
+        n = int(len(src_node_ids))
+        if not (len(dst_node_ids) == len(edge_ids) == len(node_interact_times) == n):
+            raise ValueError('src, dst, edge id and time arrays must have the same length')
+        if n == 0:
+            return
+        host = [not isinstance(a, torch.Tensor) for a in (src_node_ids, dst_node_ids, node_interact_times)]
+        if host[0] or host[1]:
+            for a, h in zip((src_node_ids, dst_node_ids), host):
+                if h:
+                    ids = np.asarray(a)
+                    if ids.min() < 0 or ids.max() >= self.num_nodes:
+                        raise IndexError(f'node id out of range for a sampler over {self.num_nodes} nodes')
+        if host[2]:
+            t = np.asarray(node_interact_times, dtype=np.float64)
+            if (n > 1 and bool((np.diff(t) < 0).any())) or t[0] < self._last_host:
+                raise ValueError('pushed times must be non-decreasing and >= every earlier pushed time')
+            self._last_host = float(t[-1])
+        else:
+            self._last_host = -np.inf           # unknown on the host: the device checks the order
+        if n > self.max_batch:
+            self._grow(n)
+        src = self._to_device(src_node_ids, torch.int64)
+        dst = self._to_device(dst_node_ids, torch.int64)
+        eid = self._to_device(edge_ids, torch.int64)
+        t = self._to_device(node_interact_times, torch.float64)
+        rc = _lib.load().tpn_stream_sampler_push(ctypes.byref(self._c), src.data_ptr(), dst.data_ptr(), eid.data_ptr(),
+                                                 t.data_ptr(), n, self._ws.data_ptr(), self._ws.numel(), self._stream())
+        if rc:
+            _lib.check(rc, 'tpn_stream_sampler_push')
+
+    def get_historical_neighbors(self, node_ids: ArrayOrTensor, node_interact_times: ArrayOrTensor,
+                                 num_neighbors: int = 20, as_tensors: bool = False
+                                 ) -> Tuple[ArrayOrTensor, ArrayOrTensor, ArrayOrTensor]:
+        """Same call and results as ``RecentNeighborSampler.get_historical_neighbors`` over the pushed edges.
+        With numpy results the error flag is checked too (``check_errors``)."""
+        assert num_neighbors > 0, 'Number of sampled neighbors for each node should be greater than 0!'
+        if num_neighbors > self.max_neighbors:
+            raise ValueError(f'num_neighbors={num_neighbors} exceeds max_neighbors={self.max_neighbors}')
+        n = int(len(node_ids))
+        if len(node_interact_times) != n:
+            raise ValueError('node ids and times must have the same length')
+        if not isinstance(node_ids, torch.Tensor) and n:
+            ids = np.asarray(node_ids)
+            if ids.min() < 0 or ids.max() >= self.num_nodes:
+                raise IndexError(f'node id out of range for a sampler over {self.num_nodes} nodes')
+        qn = self._to_device(node_ids, torch.int64)
+        qt = self._to_device(node_interact_times, torch.float64)
+        out_n = torch.empty(n, num_neighbors, dtype=torch.int64, device=self.device)
+        out_e = torch.empty(n, num_neighbors, dtype=torch.int64, device=self.device)
+        out_t = torch.empty(n, num_neighbors, dtype=torch.float64, device=self.device)
+        if n:
+            rc = _lib.load().tpn_stream_sampler_query(ctypes.byref(self._c), qn.data_ptr(), qt.data_ptr(), n,
+                                                      int(num_neighbors), out_n.data_ptr(), out_e.data_ptr(),
+                                                      out_t.data_ptr(), self._stream())
+            if rc:
+                _lib.check(rc, 'tpn_stream_sampler_query')
+        if as_tensors:
+            return out_n, out_e, out_t
+        res = out_n.cpu().numpy(), out_e.cpu().numpy(), out_t.cpu().numpy()
+        self.check_errors()
+        return res
+
+    def check_errors(self) -> None:
+        """Synchronises; raises (and clears the flag) if a device-resident input was flagged since the last check:
+        IndexError for a node id outside [0, num_nodes), ValueError for a pushed time out of order or a query before
+        the node's newest time of the previous batches."""
+        code = int(self._err.item())
+        if code == 0:
+            return
+        self._err.zero_()
+        if code & _lib.STREAM_ERR_INDEX:
+            raise IndexError(f'node id out of range for a sampler over {self.num_nodes} nodes (dropped)')
+        if code & _lib.STREAM_ERR_ORDER:
+            raise ValueError('pushed times decreased (the edge was dropped; answers are unspecified until reset())')
+        raise ValueError('a query asked for a time before the newest time its node had before the latest push: '
+                         'not answerable from the streaming state (a zero row was returned)')
 
 
 def get_neighbor_sampler(data, sample_neighbor_strategy: str = 'recent', device: Union[str, torch.device] = 'cuda:0',
