@@ -186,6 +186,11 @@ int tpn_update_phase(tpn_state_t* st,
  *                              only those above 1/4 of the call's messages; results are identical either way. */
 #define TPN_DEBUG_NO_STREAM 32
 #define TPN_DEBUG_STREAM_ALL 64
+/*   TPN_DEBUG_LEGACY_PAIRWISE: tpn_pairwise calls of more than 4,096 pairs run the one-shot TMA kernel (each warp
+ *                              stages one whole 4-pair tile and exits) instead of the persistent kernel that stages
+ *                              tiles in column halves, the next half in flight under the current one's math;
+ *                              results are identical. */
+#define TPN_DEBUG_LEGACY_PAIRWISE 128
 int tpn_set_debug_flags(int flags);
 
 
