@@ -91,6 +91,9 @@ __device__ __forceinline__ long long resolve_id(const StateView& st, long long i
 __device__ __forceinline__ float4 ld4(const float* p) { return *reinterpret_cast<const float4*>(p); }
 __device__ __forceinline__ void st4(float* p, const float4& v) { *reinterpret_cast<float4*>(p) = v; }
 
+// ReLU of the heads (torch.nn.ReLU): max(v, 0) for every number, NaN stays NaN (fmaxf would turn it into 0).
+__device__ __forceinline__ float relu(float v) { return v <= 0.f ? 0.f : v; }
+
 __device__ __forceinline__ void scale4(float4& v, float f) {
     v.x = __fmul_rn(v.x, f);
     v.y = __fmul_rn(v.y, f);

@@ -120,9 +120,9 @@ head_forward_kernel(const float* __restrict__ x, long long n, const float* __res
             for (int p = 0; p < 8; ++p) {                   // relu, H[pair][h]
                 float* row = &sm.hs[ty + 8 * p][0];
                 *reinterpret_cast<float4*>(row + tx * 4) =
-                    make_float4(fmaxf(acc[p][0].x, 0.f), fmaxf(acc[p][0].y, 0.f), fmaxf(acc[p][1].x, 0.f), fmaxf(acc[p][1].y, 0.f));
+                    make_float4(relu(acc[p][0].x), relu(acc[p][0].y), relu(acc[p][1].x), relu(acc[p][1].y));
                 *reinterpret_cast<float4*>(row + 128 + tx * 4) =
-                    make_float4(fmaxf(acc[p][2].x, 0.f), fmaxf(acc[p][2].y, 0.f), fmaxf(acc[p][3].x, 0.f), fmaxf(acc[p][3].y, 0.f));
+                    make_float4(relu(acc[p][2].x), relu(acc[p][2].y), relu(acc[p][3].x), relu(acc[p][3].y));
             }
         }
         __syncthreads();

@@ -25,6 +25,7 @@
 // (LBO = 128 B), 8-row groups 1024 B apart (SBO) — described to the tensor core by 64-bit shared-memory descriptors.
 // Every mbarrier wait is bounded (a lost arrival traps instead of hanging the GPU).
 #include <cuda_fp16.h>
+#include <float.h>
 
 #include "tpn_common.cuh"
 
@@ -52,7 +53,7 @@ struct TcSmem {
     uint64_t x_full, d1_full, d2_full, h_full[2], h_empty[2];
     uint32_t tmem_base;
     float red[8];
-    float w1_inv, w2_inv;              // 1 / (power-of-two scale of W1, W2)
+    int w1_exp, w2_exp;                // exponents of the power-of-two scales of W1, W2
 };
 
 // element (row, k) of a K = 64 operand in the canonical layout, in halfs
@@ -153,15 +154,35 @@ __device__ __forceinline__ void split8(const float (&v)[8], uint4& hi, uint4& lo
                     *reinterpret_cast<uint32_t*>(&l[2]), *reinterpret_cast<uint32_t*>(&l[3]));
 }
 
-// power-of-two scale that puts `vmax` into [2^13, 2^14): hi = fp16(v * s) is then far from fp16's overflow (2^16)
-// and lo (about 2^-11 of hi) is a normal fp16 for every element within 2^-16 of the row / matrix maximum
-__device__ __forceinline__ float pow2_scale(float vmax) {
-    if (!(vmax > 0.f) || !(vmax < 3.0e38f)) return 1.0f;
+// exponent s of the power-of-two scale 2^s that puts `vmax` into [2^13, 2^14): hi = fp16(v * 2^s) is then far from
+// fp16's overflow (2^16) and lo (about 2^-11 of hi) is a normal fp16 for every element within 2^-16 of the row /
+// matrix maximum.  s spans -114 (vmax near FLT_MAX) .. 162 (vmax = 2^-149); 0 for a zero, inf or NaN maximum.
+__device__ __forceinline__ int pow2_exp(float vmax) {
+    if (!(vmax > 0.f) || !(vmax <= FLT_MAX)) return 0;
     int e;
     (void)frexpf(vmax, &e);                                      // vmax = m * 2^e, m in [0.5, 1)
-    int s = 14 - e;
-    s = s > 100 ? 100 : (s < -100 ? -100 : s);
-    return ldexpf(1.0f, s);
+    return 14 - e;
+}
+
+// 2^s as two exact power-of-two factors, pre * post.  pre = 1 whenever 2^s is a float itself (s in [-149, 127]), so
+// one multiply (or fmaf) by `post` is the whole operation there; otherwise v * pre stays in the normal range whenever
+// v * 2^s does.  s is clamped to [-252, 254]: past that every product of the head under- or overflows anyway.
+struct Pow2 {
+    float pre, post;
+};
+__device__ __forceinline__ Pow2 pow2(int s) {
+    s = s > 254 ? 254 : (s < -252 ? -252 : s);
+    const int p = s > 127 ? s - 127 : (s < -149 ? s + 126 : 0);
+    return {ldexpf(1.0f, p), ldexpf(1.0f, s - p)};
+}
+
+// v *= f over one 64-column chunk (rare: the scale is outside the float range, see pow2)
+__device__ __forceinline__ void scale64(float (&d0)[32], float (&d1)[32], float f) {
+#pragma unroll
+    for (int j = 0; j < 32; ++j) {
+        d0[j] *= f;
+        d1[j] *= f;
+    }
 }
 
 __global__ void __launch_bounds__(kTcThreads, 1)
@@ -213,16 +234,19 @@ head_tc_kernel(const float* __restrict__ x, long long n, const float* __restrict
         __syncthreads();
         float t2 = 0.f;
         for (int wq = 0; wq < 5; ++wq) t2 = fmaxf(t2, sm.red[wq]);
-        const float s1 = pow2_scale(t1), s2 = pow2_scale(t2);
+        const int e1 = pow2_exp(t1), e2 = pow2_exp(t2);
+        const Pow2 s1 = pow2(e1), s2 = pow2(e2);
         if (tid == 0) {
-            sm.w1_inv = 1.0f / s1;        // exact: powers of two
-            sm.w2_inv = 1.0f / s2;
+            sm.w1_exp = e1;
+            sm.w2_exp = e2;
         }
         // split + canonical layout, one 16-byte K chunk (8 values) per step
         for (int c = tid; c < kHid * kF / 8; c += kTcThreads) {        // W1[h][k]: row h, chunk k8
             const int row = c >> 3, k8 = c & 7;
             const float4 a = ld4(w1 + row * kF + k8 * 8), b = ld4(w1 + row * kF + k8 * 8 + 4);
-            const float v[8] = {a.x * s1, a.y * s1, a.z * s1, a.w * s1, b.x * s1, b.y * s1, b.z * s1, b.w * s1};
+            float v[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+#pragma unroll
+            for (int j = 0; j < 8; ++j) v[j] = v[j] * s1.pre * s1.post;
             uint4 hi, lo;
             split8(v, hi, lo);
             *reinterpret_cast<uint4*>(&sm.w1[0][canon(row, k8 * 8)]) = hi;
@@ -231,7 +255,9 @@ head_tc_kernel(const float* __restrict__ x, long long n, const float* __restrict
         for (int c = tid; c < kF * kHid / 8; c += kTcThreads) {        // W2[o][h]: row o, K chunk = h / 64
             const int row = c >> 5, k8 = c & 31;
             const float4 a = ld4(w2 + row * kHid + k8 * 8), b = ld4(w2 + row * kHid + k8 * 8 + 4);
-            const float v[8] = {a.x * s2, a.y * s2, a.z * s2, a.w * s2, b.x * s2, b.y * s2, b.z * s2, b.w * s2};
+            float v[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+#pragma unroll
+            for (int j = 0; j < 8; ++j) v[j] = v[j] * s2.pre * s2.post;
             uint4 hi, lo;
             split8(v, hi, lo);
             const int kc = k8 >> 3, kk = (k8 & 7) * 8;
@@ -246,7 +272,7 @@ head_tc_kernel(const float* __restrict__ x, long long n, const float* __restrict
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem = sm.tmem_base;
-    const float w1_inv = sm.w1_inv, w2_inv = sm.w2_inv;
+    const int w1_exp = sm.w1_exp, w2_exp = sm.w2_exp;
 
     uint32_t it = 0;                      // tiles done by this CTA (phase of the once-per-tile barriers)
     if (warp < 4) {
@@ -263,13 +289,19 @@ head_tc_kernel(const float* __restrict__ x, long long n, const float* __restrict
 #pragma unroll
             for (int q = 0; q < kF / 4; ++q) xn[q] = ok ? ld4(x + row * kF + 4 * q) : make_float4(0.f, 0.f, 0.f, 0.f);
         };
-        // xn -> scaled, split, canonical layout; returns 1 / (row scale * W1 scale)
-        auto split_x = [&]() -> float {
+        // xn -> scaled, split, canonical layout; returns the exponent of 1 / (row scale * W1 scale)
+        auto split_x = [&]() -> int {
             float vmax = 0.f;
 #pragma unroll
             for (int q = 0; q < kF / 4; ++q)
                 vmax = fmaxf(vmax, fmaxf(fmaxf(fabsf(xn[q].x), fabsf(xn[q].y)), fmaxf(fabsf(xn[q].z), fabsf(xn[q].w))));
-            const float sx = pow2_scale(vmax);
+            const int ex = pow2_exp(vmax);
+            const Pow2 p = pow2(ex);
+            if (p.pre != 1.0f) {                             // rows below 2^-113: two exact steps
+#pragma unroll
+                for (int q = 0; q < kF / 4; ++q) scale4(xn[q], p.pre);
+            }
+            const float sx = p.post;
 #pragma unroll
             for (int k8 = 0; k8 < kF / 8; ++k8) {
                 const float4 a = xn[2 * k8], b = xn[2 * k8 + 1];
@@ -282,11 +314,11 @@ head_tc_kernel(const float* __restrict__ x, long long n, const float* __restrict
             fence_proxy_async_smem();
             tc_fence_before();            // this thread's TMEM reads of the previous tile are ordered before the arrival
             mbar_arrive(&sm.x_full);
-            return w1_inv / sx;                              // exact (powers of two)
+            return -(w1_exp + ex);
         };
         long long tile = blockIdx.x;
         load_x(tile);
-        float inv1 = split_x();
+        int undo1 = split_x();
         load_x(tile + gridDim.x);
         for (; tile < ntiles; tile += gridDim.x, ++it) {
             const long long row = tile * kTile + r;
@@ -295,7 +327,8 @@ head_tc_kernel(const float* __restrict__ x, long long n, const float* __restrict
             // power-of-two scale (its own row maximum), undone per chunk in epilogue 2 — no separate maximum pass
             mbar_wait_bounded(&sm.d1_full, it & 1u);
             tc_fence_after();
-            float inv2[4];
+            const Pow2 u1 = pow2(undo1);
+            int undo2[4];
 #pragma unroll 1
             for (int c = 0; c < 4; ++c) {
                 const int buf = c & 1;
@@ -304,15 +337,19 @@ head_tc_kernel(const float* __restrict__ x, long long n, const float* __restrict
                 tmem_ld32_nowait(tmem + lane_base + (uint32_t)(c * 64), d0);
                 tmem_ld32_nowait(tmem + lane_base + (uint32_t)(c * 64 + 32), d1);
                 tmem_ld_wait();
+                if (u1.pre != 1.0f) scale64(d0, d1, u1.pre);
                 float hmax = 0.f;
 #pragma unroll
                 for (int j = 0; j < 32; ++j) {
-                    d0[j] = fmaxf(fmaf(d0[j], inv1, sm.b1[c * 64 + j]), 0.f);
-                    d1[j] = fmaxf(fmaf(d1[j], inv1, sm.b1[c * 64 + 32 + j]), 0.f);
+                    d0[j] = relu(fmaf(d0[j], u1.post, sm.b1[c * 64 + j]));
+                    d1[j] = relu(fmaf(d1[j], u1.post, sm.b1[c * 64 + 32 + j]));
                     hmax = fmaxf(hmax, fmaxf(d0[j], d1[j]));
                 }
-                const float sh = pow2_scale(hmax);
-                inv2[c] = w2_inv / sh;
+                const int eh = pow2_exp(hmax);
+                const Pow2 ph = pow2(eh);
+                if (ph.pre != 1.0f) scale64(d0, d1, ph.pre);
+                const float sh = ph.post;
+                undo2[c] = -(w2_exp + eh);
                 mbar_wait_bounded(&sm.h_empty[buf], (use & 1u) ^ 1u);       // GEMM2 is done with this buffer
 #pragma unroll
                 for (int k8 = 0; k8 < 8; ++k8) {
@@ -328,9 +365,9 @@ head_tc_kernel(const float* __restrict__ x, long long n, const float* __restrict
                 mbar_arrive(&sm.h_full[buf]);
             }
             // ---- D1 is drained and GEMM1 of this tile completed long ago: hand the next tile's X to the tensor core
-            const float inv2_0 = inv2[0], inv2_1 = inv2[1], inv2_2 = inv2[2], inv2_3 = inv2[3];
+            const Pow2 u2_0 = pow2(undo2[0]), u2_1 = pow2(undo2[1]), u2_2 = pow2(undo2[2]), u2_3 = pow2(undo2[3]);
             if (tile + gridDim.x < ntiles) {
-                inv1 = split_x();
+                undo1 = split_x();
                 load_x(tile + 2 * (long long)gridDim.x);
             }
             // ---- epilogue 2: y = sum over the K chunks of D2_c / (sh_c * s2), + b2
@@ -346,9 +383,18 @@ head_tc_kernel(const float* __restrict__ x, long long n, const float* __restrict
                     tmem_ld32_nowait(tmem + lane_base + kD2Col + 128u + (uint32_t)(half * 32), d2);
                     tmem_ld32_nowait(tmem + lane_base + kD2Col + 192u + (uint32_t)(half * 32), d3);
                     tmem_ld_wait();
+                    if (u2_0.pre != 1.0f || u2_1.pre != 1.0f || u2_2.pre != 1.0f || u2_3.pre != 1.0f) {
+#pragma unroll
+                        for (int j = 0; j < 32; ++j) {
+                            d[j] *= u2_0.pre;
+                            d1[j] *= u2_1.pre;
+                            d2[j] *= u2_2.pre;
+                            d3[j] *= u2_3.pre;
+                        }
+                    }
 #pragma unroll
                     for (int j = 0; j < 32; ++j)
-                        d[j] = (d[j] * inv2_0 + d1[j] * inv2_1) + (d2[j] * inv2_2 + d3[j] * inv2_3);
+                        d[j] = (d[j] * u2_0.post + d1[j] * u2_1.post) + (d2[j] * u2_2.post + d3[j] * u2_3.post);
                 }
                 if (valid) {
 #pragma unroll

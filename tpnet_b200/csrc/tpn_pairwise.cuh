@@ -14,7 +14,7 @@ __device__ __forceinline__ float2 lo2(const float4& v) { return make_float2(v.x,
 __device__ __forceinline__ float2 hi2(const float4& v) { return make_float2(v.z, v.w); }
 
 
-// log(x) for finite x >= 1 (the epilogue only ever sees fl(max(g, 0) + 1)): exponent /
+// log(x) for finite x >= 1 (the epilogue passes NaN and +inf around it): exponent /
 // mantissa split with m in [2/3, 4/3) and a minimax polynomial for log1p(m - 1), evaluated
 // with FMAs and no special-case branches (inputs are never zero, negative, inf or denormal).
 // Checked against float64 log over [1, 1e6]: max error 0.85 ulp (torch's CPU log is <= 1 ulp).
@@ -77,6 +77,18 @@ __device__ __forceinline__ void gram_step(float2 (&acc)[R * (R + 1) / 2], const 
     }
 }
 
+// The reference's epilogue (TPNet.py:127-128): rf[rf < 0] = 0; log(rf + 1.0).  The clamp is a compare, not fmaxf,
+// so NaN stays NaN, and NaN / +inf skip the polynomial (log_ge1 is finite for them): NaN -> NaN, +inf -> +inf,
+// -inf -> 0, as torch gives.  Branch-free; finite inputs take exactly the ops of the polynomial.
+__device__ __forceinline__ float epilogue(float g, int apply_log_scale) {
+    if (apply_log_scale) {
+        const float a = __fadd_rn(g < 0.f ? 0.f : g, 1.0f);       // torch.log(x + 1.0), not log1p
+        const float r = log_ge1(a);
+        g = a < INFINITY ? r : a;
+    }
+    return g;
+}
+
 // Reduce the partial Gram sums over the G lanes of a group with a transposing butterfly
 // (each shuffle step halves the number of live values, so every lane ends up owning NP/G
 // finished entries), apply clamp + log(x + 1.0) to just those, and mirror them into the
@@ -104,11 +116,7 @@ __device__ __forceinline__ void finish_pair(const float2 (&acc)[R * (R + 1) / 2]
         if (e < NU) {
             const int rq = tab[e];
             const int r = rq >> 8, q = rq & 0xff;
-            float g = s[k];
-            if (apply_log_scale) {
-                g = fmaxf(g, 0.f);                          // random_feature[random_feature < 0] = 0
-                g = log_ge1(__fadd_rn(g, 1.0f));            // torch.log(x + 1.0), not log1p
-            }
+            const float g = epilogue(s[k], apply_log_scale);
             mine[r * R + q] = g;
             mine[q * R + r] = g;
         }

@@ -71,14 +71,6 @@ __device__ __forceinline__ void nbr_step(float2 (&acc)[H * (H + 1) / 2 + 2 * H *
     }
 }
 
-__device__ __forceinline__ float epilogue(float g, int apply_log_scale) {
-    if (apply_log_scale) {
-        g = fmaxf(g, 0.f);                          // random_feature[random_feature < 0] = 0
-        g = log_ge1(__fadd_rn(g, 1.0f));            // torch.log(x + 1.0), not log1p
-    }
-    return g;
-}
-
 template <int LAYERS, bool LAZY>
 __global__ void __launch_bounds__(kNbrMaxWarps * 32, LAYERS <= 3 ? 3 : 2)
 pairwise_nbr_kernel(StateView st, const long long* __restrict__ nbr, const long long* __restrict__ src,
