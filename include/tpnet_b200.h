@@ -59,7 +59,7 @@
 extern "C" {
 #endif
 
-#define TPN_ABI_VERSION 13
+#define TPN_ABI_VERSION 14
 
 #define TPN_MAX_LAYERS 4
 
@@ -487,6 +487,47 @@ int tpn_peer_free(void* p);
 int tpn_ipc_export(const void* p, unsigned char* handle64);
 int tpn_ipc_open(const unsigned char* handle64, void** out);
 int tpn_ipc_close(void* p);
+
+/*
+ * ---------------------------------------------------------------------------------------------------------
+ * Node-sharded streaming sampler (no reference counterpart — the reference is single-device).  The lists of node u
+ * (ALL, OLD, all_cnt, old_cnt, newest; see tpn_stream_sampler_t) live on rank u % world at local row u / world, the
+ * state's placement rule; rows [num_local_rows, num_local_rows + ext_rows) of a rank's list tables cache other
+ * ranks' lists.  The pushed batch is replicated on every rank and EVERY rank keeps all of it pending (sorted by global
+ * id), so a query never needs a remote pending entry; a push folds only the segments of the nodes the rank owns.
+ * A query call is routed like the state's node-list calls: tpn_route_nodes on `shard` (own row, or a cache slot of
+ * the sampler's own mark table) -> tpn_stream_shard_pull (the new slots' lists, out of the owners' memory) ->
+ * tpn_stream_shard_query on the translated rows.  The answers are tpn_stream_sampler_query's, bit for bit.
+ * Barrier protocol (the caller's duty, tpn_peer_barrier on `shard`): one barrier between a rank's push (its fold
+ * writes its lists) and any peer's next pull, and one between the last pull of a query phase and the next push.
+ */
+#define TPN_STREAM_PEER_TABLES 9       /* per rank: all_nbr, all_eid, all_t, old_nbr, old_eid, old_t, all_cnt, old_cnt, newest */
+typedef struct tpn_stream_shard {
+    tpn_stream_sampler_t local;        /* this rank's sampler: num_nodes = the GLOBAL node count (ids, pending keys);
+                                          the list tables hold shard.num_local_rows + shard.ext_rows rows          */
+    tpn_shard_t shard;                 /* world, rank, global_nodes (== local.num_nodes, < 2^31), num_local_rows, ext_rows
+                                          (cache rows), and the sampler's OWN mark table, counters, need_nodes,
+                                          peer_flags and barrier_seq; peer_data / peer_stamps are not used           */
+    const void* const* peer_lists;     /* DEVICE array [world][TPN_STREAM_PEER_TABLES]: rank q's list tables, mapped
+                                          into this process, in the order of TPN_STREAM_PEER_TABLES                 */
+} tpn_stream_shard_t;
+
+/* Every owned and cached row empty, nothing pending, last_time = -inf, err_flag = 0, a new generation of the cache
+ * with every shard counter (the error one too) zero. */
+int tpn_stream_shard_reset(const tpn_stream_shard_t* s, void* stream);
+/* A new cache generation, then tpn_stream_sampler_push of the replicated batch with the fold restricted to the nodes
+ * this rank owns (global ids; workspace: tpn_stream_sampler_workspace_bytes). */
+int tpn_stream_shard_push(const tpn_stream_shard_t* s, const int64_t* src_dev, const int64_t* dst_dev,
+                          const int64_t* eid_dev, const double* t_dev, int64_t batch, void* ws_dev, size_t ws_bytes,
+                          void* stream);
+/* Fills the cache slots handed out by the latest tpn_route_nodes on s->shard: newest, counts and the first count
+ * entries of ALL and OLD of each slot's node, read out of its owner's tables (one warp per slot). */
+int tpn_stream_shard_pull(const tpn_stream_shard_t* s, void* stream);
+/* tpn_stream_sampler_query for the global ids q_nodes_dev[i], reading the lists at row q_rows_dev[i] (the rows
+ * tpn_route_nodes returned: local or cache slot); the pending search uses the global id. */
+int tpn_stream_shard_query(const tpn_stream_shard_t* s, const int64_t* q_nodes_dev, const int64_t* q_rows_dev,
+                           const double* q_times_dev, int64_t n, int num_neighbors, int64_t* out_nbr_dev,
+                           int64_t* out_eid_dev, double* out_times_dev, void* stream);
 
 #ifdef __cplusplus
 }

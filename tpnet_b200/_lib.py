@@ -21,7 +21,7 @@ TPN_ERR_INDEX = -6
 STAGE_RAW, STAGE_ID_WRAP, STAGE_ID = 0, 1, 2
 TPN_MAX_LAYERS = 4
 UPDATE_WHOLE, UPDATE_PREPARE, UPDATE_APPLY = 0, 1, 2
-ABI_VERSION = 13
+ABI_VERSION = 14
 
 #: every symbol include/tpnet_b200.h declares (tests assert the .so exports all of them)
 EXPORTED_SYMBOLS = (
@@ -34,11 +34,14 @@ EXPORTED_SYMBOLS = (
     'tpn_route_workspace_bytes', 'tpn_route_update', 'tpn_route_pairs', 'tpn_route_nodes', 'tpn_pull_rows',
     'tpn_peer_barrier', 'tpn_shard_new_generation', 'tpn_peer_alloc', 'tpn_peer_free', 'tpn_ipc_export', 'tpn_ipc_open',
     'tpn_ipc_close', 'tpn_stream_sampler_workspace_bytes', 'tpn_stream_sampler_reset', 'tpn_stream_sampler_push',
-    'tpn_stream_sampler_query',
+    'tpn_stream_sampler_query', 'tpn_stream_shard_reset', 'tpn_stream_shard_push', 'tpn_stream_shard_pull',
+    'tpn_stream_shard_query',
 )
 
 SHARD_CTR_NEED, SHARD_CTR_PREV, SHARD_CTR_ERROR, SHARD_COUNTERS = 0, 1, 2, 8
 STREAM_ERR_INDEX, STREAM_ERR_ORDER, STREAM_ERR_PAST = 1, 2, 4
+#: per rank, the tables of tpn_stream_shard_t.peer_lists, in this order
+STREAM_PEER_TABLES = ('all_nbr', 'all_eid', 'all_t', 'old_nbr', 'old_eid', 'old_t', 'all_cnt', 'old_cnt', 'newest')
 
 
 class TpnState(ctypes.Structure):
@@ -105,6 +108,15 @@ class TpnStreamSampler(ctypes.Structure):
     ]
 
 
+class TpnStreamShard(ctypes.Structure):
+    """Mirror of ``tpn_stream_shard_t`` (include/tpnet_b200.h)."""
+    _fields_ = [
+        ('local', TpnStreamSampler),
+        ('shard', TpnShard),
+        ('peer_lists', c_void_p),
+    ]
+
+
 class TpnError(RuntimeError):
     def __init__(self, code: int, where: str, detail: str = ''):
         self.code = code
@@ -165,6 +177,16 @@ def _declare(lib: ctypes.CDLL) -> None:
     lib.tpn_stream_sampler_query.restype = c_int
     lib.tpn_stream_sampler_query.argtypes = [POINTER(TpnStreamSampler), c_void_p, c_void_p, c_int64, c_int, c_void_p,
                                              c_void_p, c_void_p, c_void_p]
+    for name in ('tpn_stream_shard_reset', 'tpn_stream_shard_pull'):
+        fn = getattr(lib, name)
+        fn.restype = c_int
+        fn.argtypes = [POINTER(TpnStreamShard), c_void_p]
+    lib.tpn_stream_shard_push.restype = c_int
+    lib.tpn_stream_shard_push.argtypes = [POINTER(TpnStreamShard), c_void_p, c_void_p, c_void_p, c_void_p, c_int64,
+                                          c_void_p, c_size_t, c_void_p]
+    lib.tpn_stream_shard_query.restype = c_int
+    lib.tpn_stream_shard_query.argtypes = [POINTER(TpnStreamShard), c_void_p, c_void_p, c_void_p, c_int64, c_int,
+                                           c_void_p, c_void_p, c_void_p, c_void_p]
     lib.tpn_planner_create.restype = c_int
     lib.tpn_planner_create.argtypes = [POINTER(c_void_p), c_int64, c_int, c_int]
     lib.tpn_planner_destroy.restype = None

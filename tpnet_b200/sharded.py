@@ -848,52 +848,59 @@ class ShardedRandomProjection(RandomProjectionModule):
         self._h.launches += 1
         return out
 
-    def neighbor_pair_wise_gram(self, neighbor_node_ids, src_node_ids, dst_node_ids):
+    def neighbor_pair_wise_gram(self, neighbor_node_ids, src_node_ids, dst_node_ids, sliced_neighbors: bool = False):
         """The encoder's structured call (TPNet.py:313-324) without the head, on the sharded state.  ``[m, K]`` global
         neighbour ids and ``[m]`` src / dst ids, replicated on every rank; this rank computes the rows of its positional
         slice.  Returns ``(positions in the batch, [rows, K, 2, F])``, the ``(keep, feat)`` convention of
         ``pair_wise_gram``: block ``[j, k, 0]`` is the pair ``(nbr[keep[j], k], src[keep[j]])``, ``[j, k, 1]`` the pair
-        with ``dst``.  Peer data plane (or world 1); all ranks call it together."""
+        with ``dst``.  ``sliced_neighbors=True``: ``neighbor_node_ids`` holds only the ``[rows, K]`` of this rank's slice
+        (what ``ShardedStreamingSampler`` answers on this rank), src / dst stay the whole ``[m]``.  Peer data plane (or
+        world 1); all ranks call it together."""
         self._check_node_call('neighbor_pair_wise_gram')
         dev = self._require_cuda()
         if neighbor_node_ids.ndim != 2:
             raise ValueError('neighbor_node_ids must be [m, num_neighbors]')
-        m, k = int(neighbor_node_ids.shape[0]), int(neighbor_node_ids.shape[1])
+        m = int(len(src_node_ids)) if sliced_neighbors else int(neighbor_node_ids.shape[0])
+        k = int(neighbor_node_ids.shape[1])
         if len(src_node_ids) != m or len(dst_node_ids) != m:
             raise ValueError('src and dst id arrays must have one entry per row of neighbor_node_ids')
         per, lo, hi = self._row_split(m)
         n = hi - lo
+        if sliced_neighbors and int(neighbor_node_ids.shape[0]) != n:
+            raise ValueError(f'sliced_neighbors: this rank computes rows [{lo}, {hi}) of {m}, so neighbor_node_ids must '
+                             f'have {n} rows (it has {int(neighbor_node_ids.shape[0])})')
+        nbr = neighbor_node_ids if sliced_neighbors else neighbor_node_ids[lo:hi]
         keep = self._positions(lo, hi)
         resident = all(isinstance(a, torch.Tensor) and a.is_cuda for a in (neighbor_node_ids, src_node_ids, dst_node_ids))
         if self.world == 1:
             flat = neighbor_node_ids.reshape(-1)
             return keep, self._nbr_gram_rows((flat, src_node_ids, dst_node_ids), m, k)
         if resident:
-            ids = torch.cat([neighbor_node_ids[lo:hi].reshape(-1), src_node_ids[lo:hi], dst_node_ids[lo:hi]])
+            ids = torch.cat([nbr.reshape(-1), src_node_ids[lo:hi], dst_node_ids[lo:hi]])
         else:
             host = [a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a)
-                    for a in (neighbor_node_ids, src_node_ids, dst_node_ids)]
-            ids = np.concatenate([host[0][lo:hi].reshape(-1), host[1][lo:hi], host[2][lo:hi]]).astype(np.int64,
-                                                                                                        copy=False)
+                    for a in (nbr, src_node_ids, dst_node_ids)]
+            ids = np.concatenate([host[0].reshape(-1), host[1][lo:hi], host[2][lo:hi]]).astype(np.int64, copy=False)
         rows = self._route_node_rows(ids)
         nk = n * k
         return keep, self._nbr_gram_rows((rows[:nk], rows[nk:nk + n], rows[nk + n:]), n, k)
 
     def get_neighbor_pair_wise_feature(self, neighbor_node_ids, src_node_ids, dst_node_ids,
-                                       out: Optional[torch.Tensor] = None, gather: bool = False):
+                                       out: Optional[torch.Tensor] = None, gather: bool = False,
+                                       sliced_neighbors: bool = False):
         """TPNet.py:313-324 on the sharded state: ``self.mlp`` on the ``[rows*K*2, F]`` view of
         ``neighbor_pair_wise_gram``.  Returns ``(positions in the batch, [rows, K, 2F])`` for this rank's slice (``out``:
         the buffer for that slice); ``gather=True`` returns the reference's ``[m, K, 2F]`` on every rank (one
         all_gather; collective).  The gathered tensor carries no gradient: training through a sharded state needs
-        the per-rank slices."""
-        keep, g = self.neighbor_pair_wise_gram(neighbor_node_ids, src_node_ids, dst_node_ids)
+        the per-rank slices.  ``sliced_neighbors``: as in ``neighbor_pair_wise_gram``."""
+        keep, g = self.neighbor_pair_wise_gram(neighbor_node_ids, src_node_ids, dst_node_ids, sliced_neighbors)
         n, k = g.shape[0], g.shape[1]
         f = self.pair_wise_feature_dim
         flat_out = None if out is None else out.view(n * k * 2, f)
         feat = self._head(g.view(n * k * 2, f), out=flat_out).view(n, k, 2 * f)
         if not gather:
             return keep, feat
-        m = int(neighbor_node_ids.shape[0])
+        m = int(len(src_node_ids))
         return self._gather_slices(feat, self._row_split(m)[0], m)
 
     def _gather_state_rows(self, ptr: int, n: int) -> torch.Tensor:
