@@ -82,7 +82,10 @@ typedef struct tpn_state {
     int32_t  dim;           /* d, logical row width (TPNet.py:30-33,45)                        */
     int64_t  row_stride;    /* floats, multiple of 4, >= dim                                   */
     int64_t  node_stride;   /* floats, multiple of 4, >= (L+1)*row_stride                      */
-    int32_t* stamps;        /* device, [num_nodes][L] epoch of last write of layer 1..L; NULL = eager */
+    int32_t* stamps;        /* device, [num_nodes][L] epoch of last write of layer 1..L; NULL = eager.
+                               -1 = never written: that row MUST be all zero (update reads such target and source
+                               rows as zero without loading them; gather, gather_blocks and the received-row loads of
+                               tpn_update_messages read them as stored) */
     double*  decay_log;     /* device, [log_capacity][L] f64; row e = cumulative product of the
                                fp32 factors of epochs 1..e; row 0 MUST be 1.0 (caller-initialised) */
     int64_t  log_capacity;  /* rows in decay_log                                               */

@@ -175,8 +175,10 @@ class WalkProjectionOracle:
         giants = np.nonzero(counts >= self.GIANT_MIN)[0]
         small = ~np.isin(rows, giants)
         np.add.at(tgt, rows[small], msgs[small])
-        for g in giants:
-            m = msgs[rows == g]                                   # this row's messages, in order
+        order = np.argsort(rows, kind='stable')                   # each row's messages, in order
+        start = np.searchsorted(rows[order], giants)
+        for g, lo in zip(giants, start):
+            m = msgs[order[lo:lo + counts[g]]]
             acc = tgt[g].copy()
             for c0 in range(0, m.shape[0], chunk):
                 # np.add.accumulate adds one element at a time in the array's dtype (sequential fp32 adds)

@@ -17,6 +17,7 @@ import numpy as np
 import pytest
 import torch
 
+from raw_state import RawState
 from tpnet_b200 import RandomProjectionModule, _lib
 
 pytestmark = pytest.mark.gpu
@@ -27,90 +28,7 @@ UNSUPPORTED = -5
 HEAD_FFMA = 8                                    # TPN_DEBUG_HEAD_FFMA (include/tpnet_b200.h)
 
 
-# --------------------------------------------------------------------------- raw-ABI states and the reference
-class RawState:
-    """A tpn_state_t over `rows` ([N, L+1, d] float32, the values in memory) in the given layout."""
-
-    def __init__(self, rows, rs, ns, lazy=False, rng=None, epoch=6):
-        N, H, d = rows.shape
-        L = H - 1
-        assert rs % 4 == 0 and rs >= d and ns % 4 == 0 and ns >= H * rs
-        self.N, self.L, self.d, self.rs, self.ns = N, L, d, rs, ns
-        host = np.full((N + 1, ns), np.nan, np.float32)          # gap and node N: NaN
-        blk = host[:N, :H * rs].reshape(N, H, rs)
-        blk[:] = 0
-        blk[:, :, :d] = rows
-        eff = rows.astype(np.float32).copy()
-        self.stamps = self.qlog = None
-        self.epoch = 0
-        if lazy:
-            rng = rng or np.random.default_rng(0)
-            # per-epoch fp32 factors far from 1; Q[e] = product of the factors of epochs 1..e (f64), Q[0] = 1
-            fac = rng.choice(np.float32([0.5, 0.37, 0.81, 0.62, 0.9]), size=(epoch, L)).astype(np.float64)
-            q = np.vstack([np.ones((1, L)), np.cumprod(fac, axis=0)])
-            stamps = rng.integers(-1, epoch + 1, (N, L)).astype(np.int32)
-            stamps[rng.random((N, L)) < 0.3] = rng.integers(0, 2)     # gaps of several epochs
-            for l in range(1, H):
-                dead = stamps[:, l - 1] < 0                            # never written: all zero by contract
-                blk[dead, l, :] = 0
-                eff[dead, l, :] = 0
-                s = np.maximum(stamps[:, l - 1], 0)
-                f = np.where(stamps[:, l - 1] >= 0, (q[epoch, l - 1] / q[s, l - 1]).astype(np.float32), 1.0)
-                eff[:, l, :] = eff[:, l, :] * f.astype(np.float32)[:, None]     # fl32(x * fl32(Q[e] / Q[s]))
-            self.stamps = torch.from_numpy(stamps).to(DEV)
-            self.qlog = torch.from_numpy(np.ascontiguousarray(q)).to(DEV)
-            self.epoch = epoch
-            self.cum_floor = float(q.min())
-        self.eff = eff
-        self.data = torch.from_numpy(host.reshape(-1)).to(DEV)
-        self.err = torch.zeros(1, dtype=torch.int32, device=DEV)
-        self.st = _lib.TpnState(
-            data=self.data.data_ptr(), num_nodes=N, num_layer=L, dim=d, row_stride=rs, node_stride=ns,
-            stamps=None if self.stamps is None else self.stamps.data_ptr(),
-            decay_log=None if self.qlog is None else self.qlog.data_ptr(),
-            log_capacity=self.epoch + 1, epoch=self.epoch, cum_floor=self.cum_floor if lazy else 1.0,
-            err_flag=self.err.data_ptr())
-
-    def pairwise(self, a, b, log):
-        n = len(a)
-        out = torch.full((n, 4 * (self.L + 1) ** 2), -7.0, device=DEV)
-        ad, bd = (torch.from_numpy(np.asarray(x, np.int64)).to(DEV) for x in (a, b))
-        rc = _lib.load().tpn_pairwise(ctypes.byref(self.st), ad.data_ptr(), bd.data_ptr(), n, None, int(log),
-                                      out.data_ptr(), torch.cuda.current_stream().cuda_stream)
-        assert rc == 0, rc
-        torch.cuda.synchronize()
-        assert int(self.err.item()) == 0
-        return out.cpu().numpy()
-
-    def neighbors(self, nbr, src, dst, log):
-        m, K = nbr.shape
-        F = 4 * (self.L + 1) ** 2
-        out = torch.full((m, K, 2, F), -7.0, device=DEV)
-        t = [torch.from_numpy(np.ascontiguousarray(x, np.int64)).to(DEV) for x in (nbr, src, dst)]
-        rc = _lib.load().tpn_pairwise_neighbors(ctypes.byref(self.st), t[0].data_ptr(), t[1].data_ptr(),
-                                                t[2].data_ptr(), m, K, int(log), out.data_ptr(),
-                                                torch.cuda.current_stream().cuda_stream)
-        torch.cuda.synchronize()
-        if rc == 0:
-            assert int(self.err.item()) == 0
-        return rc, out.cpu().numpy()
-
-    def reference(self, a, b, exact_nonfinite=False):
-        """(G, sum |x_i y_i|) in float64 for pairs (a, b): [n, R*R] each.  Negative ids wrap."""
-        x = np.concatenate([self.eff[np.asarray(a) % self.N], self.eff[np.asarray(b) % self.N]], axis=1)
-        x = x.astype(np.float64)
-        ax = np.abs(x)
-        n = len(x)
-        if exact_nonfinite:                      # plain loops, IEEE semantics for inf * 0 and inf - inf
-            with np.errstate(invalid='ignore', over='ignore'):
-                g = np.einsum('nrd,ncd->nrc', x, x, optimize=False)
-                s = np.einsum('nrd,ncd->nrc', ax, ax, optimize=False)
-        else:
-            g = x @ x.transpose(0, 2, 1)
-            s = ax @ ax.transpose(0, 2, 1)
-        return g.reshape(n, -1), s.reshape(n, -1)
-
-
+# --------------------------------------------------------------------------- the reference bound
 def raw_bound(s, rs):
     n = rs + 8
     return n * U / (1 - n * U) * s + n * TINY
