@@ -59,7 +59,7 @@
 extern "C" {
 #endif
 
-#define TPN_ABI_VERSION 14
+#define TPN_ABI_VERSION 15
 
 #define TPN_MAX_LAYERS 4
 
@@ -295,8 +295,29 @@ int tpn_materialize(tpn_state_t* st, void* stream);
 int tpn_reset_epoch(tpn_state_t* st, void* stream);
 
 /* Zero layers 1..L of every node and all stamps; epoch <- 0 (reset_random_projections,
- * TPNet.py:135-136; P_0 is re-drawn by the caller with torch's RNG, TPNet.py:139). */
+ * TPNet.py:135-136; P_0 is re-drawn by the caller with torch's RNG, TPNet.py:139, or with tpn_init_projection). */
 int tpn_clear_walk_layers(tpn_state_t* st, void* stream);
+
+/*
+ * P_0 from a counter-based generator (no reference counterpart; the reference draws P_0 with torch's RNG,
+ * TPNet.py:58/139).  The value of node u, column c < dim depends only on (seed, draw, u, c), so a sharded state
+ * holds the bits of the one-GPU state whatever the world size.  With s = seed, k = draw:
+ *   x[0..3] = Philox4x64-10(counter = (c / 4, u, 0, 0), key = (s, k))   (the bijection of numpy's np.random.Philox)
+ *   v_i     = ((x_i >> 11) + 0.5) * 2^-53, in f64, the add rounded to nearest (exact below 2^52): uniforms in (0, 1]
+ *   Box-Muller in f64 on (v_0, v_1) and (v_2, v_3): r = sqrt(-2 log v_even), theta = 6.283185307179586 * v_odd,
+ *             z = (r cos theta, r sin theta) -> the normals of columns 4 (c / 4) + 0..3
+ *   stored    = fl32(z * (1 / sqrt(dim))), the scale in f64: N(0, 1/sqrt(d)) as TPNet.py:58 draws it.
+ * Every f64 product and sum is rounded on its own (no FMA contraction).  log / sin / cos are not correctly rounded,
+ * so another implementation of the definition can differ only where the f64 value lies within a few f64 ulps of
+ * an f32 rounding midpoint.
+ * Local row j < rows of `st` is node first_node + j * node_step (0, 1 on one GPU; rank, world on a shard, where row
+ * j of rank r is node j * world + r).  Only columns [0, dim) of layer 0 of those rows are written (the pad columns
+ * of a partial block of 4 get zero); layers 1..L, the node_stride gap and rows >= rows (a shard's cache rows) are
+ * not touched.  rows > num_nodes, node_step < 1, first_node < 0 or a node id past INT64_MAX:
+ * TPN_ERR_INVALID_ARGUMENT.  No allocation, no synchronisation: capturable in a CUDA graph.
+ */
+int tpn_init_projection(const tpn_state_t* st, int64_t rows, int64_t first_node, int64_t node_step, uint64_t seed,
+                        uint64_t draw, void* stream);
 
 /*
  * Host -> device staging of the per-call id / timestamp arrays (the reference's

@@ -8,7 +8,7 @@ from __future__ import annotations
 
 import ctypes
 import os
-from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_size_t, c_void_p
+from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_size_t, c_uint64, c_void_p
 from typing import Optional
 
 _PKG = os.path.dirname(os.path.abspath(__file__))
@@ -21,7 +21,7 @@ TPN_ERR_INDEX = -6
 STAGE_RAW, STAGE_ID_WRAP, STAGE_ID = 0, 1, 2
 TPN_MAX_LAYERS = 4
 UPDATE_WHOLE, UPDATE_PREPARE, UPDATE_APPLY = 0, 1, 2
-ABI_VERSION = 14
+ABI_VERSION = 15
 
 #: every symbol include/tpnet_b200.h declares (tests assert the .so exports all of them)
 EXPORTED_SYMBOLS = (
@@ -35,7 +35,7 @@ EXPORTED_SYMBOLS = (
     'tpn_peer_barrier', 'tpn_shard_new_generation', 'tpn_peer_alloc', 'tpn_peer_free', 'tpn_ipc_export', 'tpn_ipc_open',
     'tpn_ipc_close', 'tpn_stream_sampler_workspace_bytes', 'tpn_stream_sampler_reset', 'tpn_stream_sampler_push',
     'tpn_stream_sampler_query', 'tpn_stream_shard_reset', 'tpn_stream_shard_push', 'tpn_stream_shard_pull',
-    'tpn_stream_shard_query',
+    'tpn_stream_shard_query', 'tpn_init_projection',
 )
 
 SHARD_CTR_NEED, SHARD_CTR_PREV, SHARD_CTR_ERROR, SHARD_COUNTERS = 0, 1, 2, 8
@@ -164,6 +164,8 @@ def _declare(lib: ctypes.CDLL) -> None:
         fn = getattr(lib, name)
         fn.restype = c_int
         fn.argtypes = [POINTER(TpnState), c_void_p]
+    lib.tpn_init_projection.restype = c_int
+    lib.tpn_init_projection.argtypes = [POINTER(TpnState), c_int64, c_int64, c_int64, c_uint64, c_uint64, c_void_p]
     lib.tpn_sampler_recent.restype = c_int
     lib.tpn_sampler_recent.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int64,
                                        c_int, c_void_p, c_void_p, c_void_p, c_void_p]

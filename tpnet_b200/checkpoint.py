@@ -8,7 +8,8 @@ stores the state ONCE, one file per rank, and can be read back into any number o
 
     <dir>/<tag>.rank<r>-of-<G>.pt     torch.save of the header
         {'format', 'world', 'rank', 'global_node_num', 'dim', 'num_layer', 'now_time', 'begging_time', 'rows',
-         'mlp': state_dict of the trainable head}
+         'mlp': state_dict of the trainable head,
+         'p0': {'seed', 'draw'} of a module with a counter-based P_0 (``p0_seed``), else None; absent in older files}
     <dir>/<tag>.rank<r>-of-<G>.state  raw little-endian float32 [rows, L+1, dim], C order
                                       (row j of rank r = node j*G + r; pending lazy decay applied)
 
@@ -34,7 +35,7 @@ from __future__ import annotations
 import glob
 import os
 import re
-from typing import Callable, Dict, Iterator, List, Sequence, Tuple, Union
+from typing import Callable, Dict, Iterator, List, Optional, Sequence, Tuple, Union
 
 import numpy as np
 import torch
@@ -131,6 +132,12 @@ def _write_rows(path: str, rows: int, per: int, row_shape: Tuple[int, ...], dtyp
             fh.write(memoryview(bufs[k & 1][:hi - lo].numpy()).cast('B'))      # leading rows of a contiguous buffer
 
 
+def _p0_header(module) -> Optional[Dict[str, int]]:
+    """Seed and draw of a module whose P_0 comes from the counter-based generator (``p0_seed``), else None."""
+    seed = getattr(module, 'p0_seed', None)
+    return None if seed is None else {'seed': int(seed), 'draw': int(module.p0_draw)}
+
+
 def save_checkpoint(module, directory: str, tag: str = 'walk_state', chunk_bytes: int = DEFAULT_CHUNK_BYTES) -> str:
     """Writes this rank's header + state file (every rank of a sharded state calls it).  The state streams to disk
     in chunks of rows through two pinned host buffers (device -> host copy of chunk k+1 overlaps the write of chunk
@@ -149,7 +156,8 @@ def save_checkpoint(module, directory: str, tag: str = 'walk_state', chunk_bytes
     header = {'format': FORMAT, 'world': int(world), 'rank': int(rank), 'global_node_num': int(global_n), 'dim': int(d),
               'num_layer': int(module.num_layer), 'now_time': float(module._now_host),
               'begging_time': float(module.begging_time.item()), 'rows': int(rows),
-              'mlp': {k: v.detach().to('cpu') for k, v in module.mlp.state_dict().items()}}
+              'mlp': {k: v.detach().to('cpu') for k, v in module.mlp.state_dict().items()},
+              'p0': _p0_header(module)}
     torch.save(header, path + '.tmp')
     os.replace(spath + '.tmp', spath)
     os.replace(path + '.tmp', path)                         # the header appears last: a reader never sees half a shard
@@ -215,6 +223,10 @@ def load_checkpoint(module, directory: str, tag: str = 'walk_state', load_head: 
         module.begging_time.data.fill_(header['begging_time'])
         if load_head:
             module.mlp.load_state_dict(header['mlp'])
+        # a counter-mode module continues the saved generator: its next reset draws what the saved job's would
+        if getattr(module, 'p0_seed', None) is not None and header.get('p0') is not None:
+            module.p0_seed = int(header['p0']['seed'])
+            module.p0_draw = int(header['p0']['draw'])
     module._after_external_write()                          # host clock mirror, lazy bookkeeping restart
 
 

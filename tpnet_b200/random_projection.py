@@ -108,7 +108,7 @@ class RandomProjectionModule(nn.Module):
                  device: str, use_matrix: bool, beginning_time: np.float64, not_scale: bool, enforce_dim: int,
                  decay_mode: str = 'auto', init_p0: bool = True, state_device=None,
                  accumulation: str = 'reference', giant_chunk: int = 1024,
-                 state_buffer: Optional[torch.Tensor] = None):
+                 state_buffer: Optional[torch.Tensor] = None, p0_seed: Optional[int] = None):
         """Arguments as the reference constructor (TPNet.py:10-26).  ``decay_mode`` in
         {'auto', 'eager', 'lazy'} selects how the time decay of TPNet.py:83-85 is
         realised; all modes produce the same values.  ``init_p0=False`` leaves P_0 zero for the
@@ -121,8 +121,24 @@ class RandomProjectionModule(nn.Module):
         deterministic, within fp32 rounding of the reference order (include/tpnet_b200.h,
         ``tpn_state_t::giant_chunk``), and free of the hub's sequential add chain.  ``state_buffer``: a
         zero-filled float32 tensor ``[node_num, num_layer + 1, row_stride]`` to use as the packed state
-        (the sharded module passes peer-visible memory)."""
+        (the sharded module passes peer-visible memory).  ``p0_seed``: an int in [0, 2^64) draws P_0 on the state's
+        device from the counter-based generator of ``tpn_init_projection`` (include/tpnet_b200.h) instead of torch's
+        RNG — draw 0 here, draw ``p0_draw`` after ``p0_draw`` resets — so every placement of the rows, sharded at any
+        world size or not, holds the same bits; no torch RNG state is consumed.  Needs ``state_device`` on CUDA."""
         super().__init__()
+        if p0_seed is not None:
+            if use_matrix:
+                raise ValueError('p0_seed: use_matrix has P_0 = I, there is nothing to draw')
+            if not init_p0:
+                raise ValueError('p0_seed draws P_0: it cannot be combined with init_p0=False')
+            sdev = state_buffer.device if state_buffer is not None else (
+                torch.device(state_device) if state_device is not None else None)
+            if sdev is None or sdev.type != 'cuda':
+                raise ValueError('p0_seed draws P_0 on the GPU: create the state there with state_device')
+            if not 0 <= int(p0_seed) < 1 << 64:
+                raise ValueError('p0_seed must be in [0, 2^64)')
+        self.p0_seed = None if p0_seed is None else int(p0_seed)
+        self.p0_draw = 0
         if not 1 <= num_layer <= _lib.TPN_MAX_LAYERS:
             raise ValueError(f'num_layer must be in 1..{_lib.TPN_MAX_LAYERS}')
         if decay_mode not in ('auto', 'eager', 'lazy'):
@@ -164,7 +180,7 @@ class RandomProjectionModule(nn.Module):
                                       device=state_device)
         if self.use_matrix:
             self._state[:, 0, :self.dim] = torch.eye(self.node_num)      # TPNet.py:48-49
-        elif init_p0:
+        elif init_p0 and self.p0_seed is None:
             # same RNG call as TPNet.py:58 so a seeded run draws the same P_0
             self._state[:, 0, :self.dim] = torch.normal(0, 1 / math.sqrt(self.dim), (self.node_num, self.dim))
         self.random_projections = nn.ParameterList(
@@ -191,6 +207,8 @@ class RandomProjectionModule(nn.Module):
         self.fused_head = True          # no-grad calls: fused fp32 head kernel when the head has the default shape
         self.register_state_dict_pre_hook(lambda module, prefix, keep_vars: module.materialize())
         self.register_load_state_dict_post_hook(lambda module, incompatible: module._after_external_write())
+        if self.p0_seed is not None:
+            self._write_counter_p0()
 
     # ------------------------------------------------------------------ plumbing
     @property
@@ -602,17 +620,41 @@ class RandomProjectionModule(nn.Module):
         self._h.epoch = 0
         self._h.now = self._h.begin
         self.now_time.data.copy_(self.begging_time.data)     # in place: the parameter keeps its storage (CUDA graphs)
-        if not self.use_matrix:
-            std = 1 / math.sqrt(self.dim)
-            p0 = self.random_projections[0]
-            with torch.no_grad():
-                if self.node_num * self.dim * 4 <= (2 << 30):
-                    # draw into a contiguous [N, d] tensor exactly like nn.init.normal_ on the
-                    # reference's contiguous parameter (same generator stream), then place it
-                    p0.copy_(torch.empty(self.node_num, self.dim, dtype=torch.float32, device=p0.device)
-                             .normal_(mean=0, std=std))
-                else:
-                    p0.normal_(mean=0, std=std)
+        if self.use_matrix:
+            return
+        if self.p0_seed is not None:
+            self.p0_draw += 1
+            self._write_counter_p0()
+            return
+        self._redraw_p0()
+
+    def _redraw_p0(self) -> None:
+        """P_0 of a reset drawn with torch's RNG (TPNet.py:139)."""
+        std = 1 / math.sqrt(self.dim)
+        p0 = self.random_projections[0]
+        with torch.no_grad():
+            if self.node_num * self.dim * 4 <= (2 << 30):
+                # draw into a contiguous [N, d] tensor exactly like nn.init.normal_ on the
+                # reference's contiguous parameter (same generator stream), then place it
+                p0.copy_(torch.empty(self.node_num, self.dim, dtype=torch.float32, device=p0.device)
+                         .normal_(mean=0, std=std))
+            else:
+                p0.normal_(mean=0, std=std)
+
+    def _p0_rows(self) -> Tuple[int, int, int]:
+        """(rows, first node, node step) of the P_0 rows this module owns: all of them, node j at row j."""
+        return self.node_num, 0, 1
+
+    def _write_counter_p0(self) -> None:
+        """Draw ``p0_draw`` of the counter-based generator into the owned rows of P_0 (tpn_init_projection)."""
+        self._require_cuda()
+        rows, first, step = self._p0_rows()
+        # a layout-only view: the kernel reads no stamps, and the module's cached C state is left alone
+        st = TpnState(data=self._state.data_ptr(), num_nodes=self.node_num, num_layer=self.num_layer, dim=self.dim,
+                      row_stride=self.row_stride, node_stride=self.node_stride)
+        rc = _lib.load().tpn_init_projection(ctypes.byref(st), rows, first, step, self.p0_seed, self.p0_draw,
+                                             self._stream())
+        _lib.check(rc, 'tpn_init_projection')
 
     def backup_random_projections(self) -> Tuple[torch.Tensor, List[torch.Tensor]]:
         """TPNet.py:141-147: (now_time, [P_1..P_L]) — P_0 is not part of the backup."""

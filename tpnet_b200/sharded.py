@@ -193,15 +193,24 @@ class ShardedRandomProjection(RandomProjectionModule):
     ``group`` when torch.distributed is initialised; ``LocalPeerGroup`` views put several ranks in one
     process).  ``route_cap_factor`` bounds the share of a call's items one rank may own (the launches of the
     rank-local kernels are sized for ``min(1, factor / world)`` of the call; an overflow is flagged, never silent).
+
+    P_0: ``p0='global'`` draws the whole ``[N, d]`` matrix on the host and keeps this rank's rows (the one-GPU values
+    under the same torch seed); any other value leaves it to ``init_p0_on_device`` (per-rank seeds: the values depend
+    on the world size).  ``p0_seed`` (with the default ``p0``): the counter-based generator of ``tpn_init_projection``
+    writes this rank's rows on its GPU, the same bits as the one-GPU module with the same ``p0_seed`` at any world
+    size, at construction and after every reset.
     """
 
     def __init__(self, node_num: int, edge_num: int, dim_factor: int, num_layer: int, time_decay_weight: float,
                  device: str, use_matrix: bool, beginning_time: np.float64, not_scale: bool, enforce_dim: int,
                  decay_mode: str = 'lazy', group=None, ext_rows: int = 1 << 16, p0: str = 'global',
                  state_device=None, exchange: str = 'auto', peers: Optional[PeerGroup] = None,
-                 route_cap_factor: float = 3.5, accumulation: str = 'reference', giant_chunk: int = 1024):
+                 route_cap_factor: float = 3.5, accumulation: str = 'reference', giant_chunk: int = 1024,
+                 p0_seed: Optional[int] = None):
         if use_matrix:
             raise ValueError('use_matrix keeps N x N matrices: not meaningful for a sharded state')
+        if p0_seed is not None and p0 != 'global':
+            raise ValueError("p0_seed selects the counter-based P_0: leave p0 at its default")
         if exchange not in ('auto', 'peer', 'nccl'):
             raise ValueError("exchange must be 'auto', 'peer' or 'nccl'")
         self.group = group
@@ -223,7 +232,7 @@ class ShardedRandomProjection(RandomProjectionModule):
         # the width rule uses the GLOBAL node count (TPNet.py:30-33)
         dim = enforce_dim if enforce_dim != -1 else min(int(math.log(edge_num * 2)) * dim_factor, node_num)
         self._p0_mode = p0
-        if p0 == 'global':
+        if p0 == 'global' and p0_seed is None:
             # draw the global P_0 exactly like the single-GPU module and keep this rank's rows:
             # same values as an unsharded run with the same seed (parity tests)
             full = torch.normal(0, 1 / math.sqrt(dim), (self.global_node_num, dim))
@@ -246,8 +255,8 @@ class ShardedRandomProjection(RandomProjectionModule):
         super().__init__(node_num=self.n_local + self.ext_rows, edge_num=edge_num, dim_factor=dim_factor,
                          num_layer=num_layer, time_decay_weight=time_decay_weight, device=device, use_matrix=False,
                          beginning_time=beginning_time, not_scale=not_scale, enforce_dim=dim, decay_mode=decay_mode,
-                         init_p0=False, state_device=state_device, accumulation=accumulation, giant_chunk=giant_chunk,
-                         state_buffer=state_buffer)
+                         init_p0=p0_seed is not None, state_device=state_device, accumulation=accumulation,
+                         giant_chunk=giant_chunk, state_buffer=state_buffer, p0_seed=p0_seed)
         with torch.no_grad():
             if mine is not None:
                 self.random_projections[0][:self.n_local].copy_(mine)
@@ -282,6 +291,23 @@ class ShardedRandomProjection(RandomProjectionModule):
             for lo in range(0, self.n_local, block):
                 hi = min(lo + block, self.n_local)
                 p0[lo:hi].copy_(torch.randn(hi - lo, self.dim, device=p0.device, generator=g) / math.sqrt(self.dim))
+
+    def _p0_rows(self) -> Tuple[int, int, int]:
+        return self.n_local, self.rank, self.world             # row j is node j * world + rank; cache rows untouched
+
+    def _redraw_p0(self) -> None:
+        """P_0 of a reset with torch's RNG, own rows only (the cache rows are stale until the next pull anyway).
+        'global': the one-GPU module's draw from the same generator state (its contiguous [N, d] draw), rows
+        rank::world of it — every rank seeded alike draws the reset of the unsharded run.  'device': one seed from
+        torch's default generator, then ``init_p0_on_device`` of it, so the ranks draw different rows."""
+        if self._p0_mode == 'global':
+            std = 1 / math.sqrt(self.dim)
+            with torch.no_grad():
+                full = torch.empty(self.global_node_num, self.dim, dtype=torch.float32,
+                                   device=self._state.device).normal_(mean=0, std=std)
+                self.random_projections[0][:self.n_local].copy_(full[self.rank::self.world])
+        else:
+            self.init_p0_on_device(int(torch.randint(0, 1 << 31, (1,)).item()))
 
     def _ext_view(self, rows: int) -> torch.Tensor:
         if rows > self.ext_rows:
