@@ -178,10 +178,6 @@ def single_gpu(shape_name, args, dev):
         groups = LocalPeerGroup.create(world)
         ranks = [sharded_module(sh, dev, world, r, groups[r]) for r in range(world)]
         for m in ranks:
-            for name in ('state', 'stamps', 'flags'):
-                if name in m._peer_bufs:
-                    m._peers.publish(name, m._peer_bufs[name])
-        for m in ranks:
             m.connect()
         for s, d, t in batches:
             pend = [m.update_begin(s, d, t) for m in ranks]
@@ -192,7 +188,7 @@ def single_gpu(shape_name, args, dev):
         calls, store = [], {}
         k = sh['K']
         for m in ranks:
-            per, lo, hi = m._row_split(sh['m'])
+            per, lo, hi = m.row_split(sh['m'])
             n = hi - lo
             ids = torch.cat([nbr[lo:hi].reshape(-1), src[lo:hi], dst[lo:hi]])
 
@@ -221,7 +217,7 @@ def single_gpu(shape_name, args, dev):
             m.check_errors()
         out[f'in_process_world{world}'] = {
             'note': 'all ranks on one GPU, one after the other: pulls read local HBM, not NVLink',
-            'rows_per_rank': [m._row_split(sh['m'])[2] - m._row_split(sh['m'])[1] for m in ranks],
+            'rows_per_rank': [m.row_split(sh['m'])[2] - m.row_split(sh['m'])[1] for m in ranks],
             'rows_pulled_per_call': pulled, 'times': {k2: stats(v) for k2, v in res.items()}}
         del ranks, calls, store
         torch.cuda.empty_cache()

@@ -73,7 +73,7 @@ def ms(pairs):
 
 def sampler_bytes(s):
     ts = list(s._lists.values()) + [s._all_cnt, s._old_cnt, s._newest, s._ws] + list(s._pend.values())
-    ts += [getattr(s, k) for k in ('_mark', '_need') if hasattr(s, k)]
+    ts += [s._shard_tensors[k] for k in ('mark', 'need') if k in s._shard_tensors]
     return int(sum(t.numel() * t.element_size() for t in ts))
 
 
@@ -146,7 +146,7 @@ def in_process(args, dev, world):
             for r, s in enumerate(ranks):
                 push[r].append(pe[r][0].elapsed_time(pe[r][1]))
                 query[r].append(qe[r][0].elapsed_time(qe[r][1]))
-                pulled[r].append(int(s._counters[_lib.SHARD_CTR_NEED].item()))
+                pulled[r].append(int(s._shard_tensors['counters'][_lib.SHARD_CTR_NEED].item()))
     for s in ranks:
         s.check_errors()
     out = {'world': world, 'num_nodes': N, 'batch': B, 'K': K, 'cache_rows': args.cache_rows,
@@ -177,7 +177,7 @@ def distributed(args):
         if i >= args.warm:
             push.append(p[0].elapsed_time(p[1]))
             query.append(q[0].elapsed_time(q[1]))
-            pulled.append(int(s._counters[_lib.SHARD_CTR_NEED].item()))
+            pulled.append(int(s._shard_tensors['counters'][_lib.SHARD_CTR_NEED].item()))
     s.check_errors()
     mine = dict(per_rank_summary(push, query, pulled), rank=rank, n_local=s.n_local,
                 table_bytes=(s.n_local + s.cache_rows) * (48 * K + 16), device_bytes=sampler_bytes(s))

@@ -27,7 +27,7 @@ TPN_ERR_INVALID_ARGUMENT = -1
 # ---------------------------------------------------------------- in-process ranks (as in tests/test_gpu_sharded.py)
 @pytest.fixture
 def local_ranks():
-    """Factory of in-process ranks on cuda:0: every buffer published, every rank connected; each rank has a stream.
+    """Factory of in-process ranks on cuda:0: every rank connected; each rank has a stream.
     World 1 is the sharded class without peers (its whole graph is local)."""
     from tpnet_b200.peer import LocalPeerGroup
     from tpnet_b200.sharded import ShardedRandomProjection
@@ -40,11 +40,6 @@ def local_ranks():
             ranks.append(ShardedRandomProjection(decay_mode=mode, ext_rows=ext_rows, peers=groups[r],
                                                  exchange='peer' if world > 1 else 'auto', state_device=DEV,
                                                  **extra, **kw).to(DEV))
-        for m in ranks if world > 1 else ():
-            m._peers.publish('state', m._peer_bufs['state'])
-            if 'stamps' in m._peer_bufs:
-                m._peers.publish('stamps', m._peer_bufs['stamps'])
-            m._peers.publish('flags', m._peer_bufs['flags'])
         for m in ranks:
             m.connect()
         return ranks, [torch.cuda.Stream() for _ in range(world)]

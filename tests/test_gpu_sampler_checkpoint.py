@@ -302,10 +302,6 @@ def _job(world, N, K, B, mode):
             torch.manual_seed(11)                  # p0='global': every rank draws the same global P_0, keeps its rows
             states.append(ShardedRandomProjection(ext_rows=2 * N + 64, peers=groups[r], exchange='peer', **kw).to(DEV))
         for m in states:
-            for name in ('state', 'stamps', 'flags'):
-                if name in m._peer_bufs:
-                    m._peers.publish(name, m._peer_bufs[name])
-        for m in states:
             m.connect()
         samplers, _ = make_ranks(world, N, K, B, N)
     return list(zip(samplers, states)), [torch.cuda.Stream() for _ in range(world)]

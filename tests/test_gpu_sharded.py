@@ -72,11 +72,6 @@ def _sim_ranks(world, kw, mode, ext_rows, accumulation='reference', chunk=1024):
                                              state_device='cuda:0', accumulation=accumulation, giant_chunk=chunk,
                                              **kw).to('cuda:0'))
     for m in ranks:
-        m._peers.publish('state', m._peer_bufs['state'])          # every buffer is published before anyone connects
-        if 'stamps' in m._peer_bufs:
-            m._peers.publish('stamps', m._peer_bufs['stamps'])
-        m._peers.publish('flags', m._peer_bufs['flags'])
-    for m in ranks:
         m.connect()
     return ranks, [torch.cuda.Stream() for _ in range(world)]
 

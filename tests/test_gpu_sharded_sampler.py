@@ -287,9 +287,6 @@ def _state_ranks(world, N):
         ranks.append(ShardedRandomProjection(decay_mode='lazy', ext_rows=2 * N + 64, peers=groups[r], exchange='peer',
                                              state_device=DEV, **_state_kw(N)).to(DEV))
     for m in ranks:
-        for name in ('state', 'stamps', 'flags'):
-            m._peers.publish(name, m._peer_bufs[name])
-    for m in ranks:
         m.connect()
     torch.manual_seed(11)
     ref = RandomProjectionModule(decay_mode='lazy', **_state_kw(N)).to(DEV)

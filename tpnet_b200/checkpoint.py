@@ -40,7 +40,7 @@ from typing import Callable, Dict, Iterator, List, Optional, Sequence, Tuple, Un
 import numpy as np
 import torch
 
-from .sharded import rows_on_rank
+from .peer import rows_on_rank
 
 FORMAT_V1 = 'tpnet_b200.shard.v1'
 FORMAT = 'tpnet_b200.shard.v2'
@@ -48,13 +48,10 @@ SAMPLER_FORMAT = 'tpnet_b200.sampler.v1'
 DEFAULT_CHUNK_BYTES = 64 << 20
 
 
-def _shard_info(module) -> Tuple[int, int, int, int]:
-    """(world, rank, rows owned by this rank, global node count) of a plain or sharded module."""
-    world = int(getattr(module, 'world', 1))
-    rank = int(getattr(module, 'rank', 0))
-    rows = int(getattr(module, 'n_local', module.node_num))
-    global_n = int(getattr(module, 'global_node_num', module.node_num))
-    return world, rank, rows, global_n
+def _shard_info(obj, num_nodes: int) -> Tuple[int, int, int]:
+    """(world, rank, rows this rank owns) of a plain or sharded state or sampler over ``num_nodes`` nodes; cache rows
+    are not owned."""
+    return int(getattr(obj, 'world', 1)), int(getattr(obj, 'rank', 0)), int(getattr(obj, 'n_local', num_nodes))
 
 
 def shard_path(directory: str, tag: str, rank: int, world: int) -> str:
@@ -64,7 +61,7 @@ def shard_path(directory: str, tag: str, rank: int, world: int) -> str:
 def pack_shard(state_rows: torch.Tensor, world: int, rank: int, global_node_num: int, now_time: float,
                begging_time: float, head: Dict[str, torch.Tensor]) -> dict:
     """Payload of one rank.  ``state_rows``: float32 [rows, L+1, dim] of the nodes rank, rank+world, ..."""
-    rows_expected = (global_node_num - rank + world - 1) // world if global_node_num > rank else 0
+    rows_expected = rows_on_rank(global_node_num, world, rank)
     if state_rows.dim() != 3 or state_rows.shape[0] != rows_expected or state_rows.dtype != torch.float32:
         raise ValueError(f'rank {rank} of {world} owns {rows_expected} of {global_node_num} nodes; got state '
                          f'{tuple(state_rows.shape)} {state_rows.dtype}')
@@ -144,7 +141,8 @@ def save_checkpoint(module, directory: str, tag: str = 'walk_state', chunk_bytes
     k).  Returns the header path."""
     os.makedirs(directory, exist_ok=True)
     module.materialize()                                    # lazy decay: bring every row current first
-    world, rank, rows, global_n = _shard_info(module)
+    global_n = int(getattr(module, 'global_node_num', module.node_num))
+    world, rank, rows = _shard_info(module, global_n)
     L1, d = module.num_layer + 1, module.dim
     path = shard_path(directory, tag, rank, world)
     spath = state_path(path)
@@ -188,7 +186,8 @@ def load_checkpoint(module, directory: str, tag: str = 'walk_state', load_head: 
                     chunk_bytes: int = DEFAULT_CHUNK_BYTES) -> None:
     """Reads a checkpoint written with ANY number of ranks into this module's rows (re-sharding by node id:
     a single-GPU state can be loaded into 8 shards and back).  State files are memory-mapped and copied in chunks."""
-    world, rank, rows, global_n = _shard_info(module)
+    global_n = int(getattr(module, 'global_node_num', module.node_num))
+    world, rank, rows = _shard_info(module, global_n)
     total = 0
     header = None
     with torch.no_grad():
@@ -257,13 +256,6 @@ def _sampler_tables(sampler) -> List[torch.Tensor]:
     return [sampler._lists[k] for k in _LIST_FIELDS] + [sampler._all_cnt, sampler._old_cnt, sampler._newest]
 
 
-def _sampler_info(sampler) -> Tuple[int, int, int]:
-    """(world, rank, rows this rank owns) of a plain or sharded sampler; cache rows are not owned."""
-    world = int(getattr(sampler, 'world', 1))
-    rank = int(getattr(sampler, 'rank', 0))
-    return world, rank, int(getattr(sampler, 'n_local', sampler.num_nodes))
-
-
 def _record_fields(chunk: torch.Tensor, tables: Sequence[torch.Tensor]) -> List[torch.Tensor]:
     """Views of a uint8 [m, 48 C + 16] block of records, one per table (the table's dtype and row shape)."""
     out, off = [], 0
@@ -281,7 +273,7 @@ def save_sampler(sampler, directory: str, tag: str = 'sampler', chunk_bytes: int
     host buffers of ``chunk_bytes``.  A sampler with a flagged device error raises (``check_errors``) before anything
     is written: its answers are unspecified.  Returns the header path."""
     sampler.check_errors()
-    world, rank, rows = _sampler_info(sampler)
+    world, rank, rows = _shard_info(sampler, sampler.num_nodes)
     C = int(sampler.max_neighbors)
     rb = sampler_row_bytes(C)
     os.makedirs(directory, exist_ok=True)
@@ -364,7 +356,7 @@ def load_sampler(sampler, directory: str, tag: str = 'sampler', chunk_bytes: int
     the next push and queries answer exactly as the saved sampler's would.  The tables are written in place, so a
     CUDA graph captured on this sampler before the load stays valid, unless the pending batch exceeds
     ``2 * max_batch``: then the pending buffers grow, which is refused inside a capture."""
-    world, rank, rows = _sampler_info(sampler)
+    world, rank, rows = _shard_info(sampler, sampler.num_nodes)
     C = int(sampler.max_neighbors)
     rb = sampler_row_bytes(C)
     shards = sampler_shards(directory, tag, int(sampler.num_nodes), C)

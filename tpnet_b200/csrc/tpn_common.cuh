@@ -75,6 +75,35 @@ inline int validate_state(const tpn_state_t* st) {
 void set_cuda_error(cudaError_t e);
 int check_launch();
 
+// ---------------------------------------------------------------- routing shard (tpn_shard_t), tpn_route.cu and tpn_sampler.cu
+inline int validate_shard(const tpn_shard_t* sh) {
+    if (sh == nullptr || sh->world < 1 || sh->world > 64 || sh->rank < 0 || sh->rank >= sh->world ||
+        sh->global_nodes < 1 || sh->global_nodes > 0x7fffffffll || sh->num_local_rows < 0 || sh->ext_rows < 0 ||
+        sh->ext_rows > 0x7ffffff0ll || sh->mark == nullptr || sh->counters == nullptr || sh->need_nodes == nullptr)
+        return TPN_ERR_INVALID_ARGUMENT;
+    return TPN_OK;
+}
+
+// A new cache generation after a write: every mark cleared, NEED and PREV restart; the error counter is sticky until
+// the host reads it.
+inline int shard_new_generation(const tpn_shard_t* sh, cudaStream_t stream) {
+    cudaError_t e = cudaMemsetAsync(sh->mark, 0, sizeof(int32_t) * (size_t)sh->global_nodes, stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(sh->counters, 0, sizeof(int32_t) * 2, stream);
+    if (e != cudaSuccess) {
+        set_cuda_error(e);
+        return TPN_ERR_CUDA;
+    }
+    return TPN_OK;
+}
+
+// The cache slots the latest routing call handed out, [counters[PREV], min(counters[NEED], ext_rows)): a pull fills
+// exactly these.
+__device__ __forceinline__ void new_slots(const int* counters, long long ext_rows, int& first, int& last) {
+    first = counters[TPN_SHARD_CTR_PREV];
+    const int need = counters[TPN_SHARD_CTR_NEED];
+    last = need < ext_rows ? need : (int)ext_rows;
+}
+
 // Device-resident node id -> row.  Indexing calls (pair-wise, gather: TPNet.py:109 indexes tensors, where
 // negative ids wrap) pass wrap = true.  An id outside the range is the reference's IndexError: it cannot be
 // raised from a kernel, so the flag is set (RandomProjectionModule.check_errors raises) and the id is

@@ -266,9 +266,8 @@ __global__ void __launch_bounds__(256)
 pull_rows_kernel(StateView st, ShardView sh, int ds4) {
     const int lane = threadIdx.x & 31;
     const int warps = gridDim.x * (blockDim.x >> 5);
-    const int first = sh.counters[TPN_SHARD_CTR_PREV];
-    int last = sh.counters[TPN_SHARD_CTR_NEED];
-    last = last < sh.ext_rows ? last : (int)sh.ext_rows;
+    int first, last;
+    new_slots(sh.counters, sh.ext_rows, first, last);
     const int L = st.num_layer;
     const int rows4 = (L + 1) * ds4;
     for (int slot = first + blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); slot < last; slot += warps) {
@@ -341,14 +340,6 @@ peer_barrier_kernel(ShardView sh, long long spin_limit) {
     __syncthreads();
     __threadfence_system();
     if (threadIdx.x == 0) *sh.barrier_seq = seq;
-}
-
-int validate_shard(const tpn_shard_t* sh) {
-    if (sh == nullptr || sh->world < 1 || sh->world > 64 || sh->rank < 0 || sh->rank >= sh->world ||
-        sh->global_nodes < 1 || sh->global_nodes > 0x7fffffffll || sh->num_local_rows < 0 || sh->ext_rows < 0 ||
-        sh->ext_rows > 0x7ffffff0ll || sh->mark == nullptr || sh->counters == nullptr || sh->need_nodes == nullptr)
-        return TPN_ERR_INVALID_ARGUMENT;
-    return TPN_OK;
 }
 
 int route_impl(const tpn_shard_t* sh, const Items& it, int64_t* first_rows, int64_t* second_rows, int64_t* keep,
@@ -475,15 +466,7 @@ extern "C" int tpn_shard_new_generation(const tpn_shard_t* sh, void* stream_v) {
     int rc = validate_shard(sh);
     if (rc != TPN_OK) return rc;
     DeviceScope scope(sh->mark);
-    cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_v);
-    cudaError_t e = cudaMemsetAsync(sh->mark, 0, sizeof(int32_t) * (size_t)sh->global_nodes, stream);
-    // NEED and PREV restart; the error counter is sticky until the host reads it
-    if (e == cudaSuccess) e = cudaMemsetAsync(sh->counters, 0, sizeof(int32_t) * 2, stream);
-    if (e != cudaSuccess) {
-        set_cuda_error(e);
-        return TPN_ERR_CUDA;
-    }
-    return TPN_OK;
+    return shard_new_generation(sh, reinterpret_cast<cudaStream_t>(stream_v));
 }
 
 // ---------------------------------------------------------------- peer-visible memory (CUDA IPC)

@@ -334,9 +334,8 @@ stream_pull_kernel(StreamView v, const void* const* __restrict__ peer, const int
                    const long long* __restrict__ need_nodes, long long n_local, long long ext_rows) {
     const int lane = threadIdx.x & 31;
     const int warps = gridDim.x * (blockDim.x >> 5);
-    const int first = counters[TPN_SHARD_CTR_PREV];
-    int last = counters[TPN_SHARD_CTR_NEED];
-    last = last < ext_rows ? last : (int)ext_rows;
+    int first, last;
+    new_slots(counters, ext_rows, first, last);
     for (int slot = first + blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); slot < last; slot += warps) {
         const long long u = need_nodes[slot];
         const void* const* T = peer + (u % v.world) * TPN_STREAM_PEER_TABLES;
@@ -401,17 +400,16 @@ bool stream_tables_set(const tpn_stream_sampler_t* s) {
            s->pend_t != nullptr && s->pend_count != nullptr && s->last_time != nullptr && s->err_flag != nullptr;
 }
 
-// A sharded sampler: the plain checks, a shard whose placement matches the global node count (so every row a kernel
-// computes is inside the tables), and the sampler's own routing tables.
+// A sharded sampler: the plain checks, the shard's, and a placement that matches the sampler's node count (so every
+// row a kernel computes is inside the tables).
 int validate_stream_shard(const tpn_stream_shard_t* s) {
     if (s == nullptr) return TPN_ERR_INVALID_ARGUMENT;
-    const int rc = validate_stream(&s->local);
+    int rc = validate_stream(&s->local);
+    if (rc == TPN_OK) rc = validate_shard(&s->shard);
     if (rc != TPN_OK) return rc;
     const tpn_shard_t& h = s->shard;
-    if (h.world < 1 || h.world > 64 || h.rank < 0 || h.rank >= h.world || h.global_nodes != s->local.num_nodes ||
-        h.global_nodes > 0x7fffffffll || h.ext_rows < 0 || h.ext_rows > 0x7ffffff0ll ||
-        h.num_local_rows != (h.global_nodes > h.rank ? (h.global_nodes - h.rank + h.world - 1) / h.world : 0) ||
-        h.mark == nullptr || h.counters == nullptr || h.need_nodes == nullptr)
+    if (h.global_nodes != s->local.num_nodes ||
+        h.num_local_rows != (h.global_nodes > h.rank ? (h.global_nodes - h.rank + h.world - 1) / h.world : 0))
         return TPN_ERR_INVALID_ARGUMENT;
     return TPN_OK;
 }
@@ -579,14 +577,9 @@ extern "C" int tpn_stream_shard_push(const tpn_stream_shard_t* s, const int64_t*
     if (rc != TPN_OK || !launch) return rc;
     DeviceScope scope(s->local.newest);
     cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_v);
-    // the fold rewrites lists that other ranks may hold in their caches, and this rank's cache is of the old lists:
-    // a new generation (NEED and PREV restart; the error counter is sticky until the host reads it)
-    cudaError_t e = cudaMemsetAsync(s->shard.mark, 0, sizeof(int32_t) * (size_t)s->shard.global_nodes, stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(s->shard.counters, 0, sizeof(int32_t) * 2, stream);
-    if (e != cudaSuccess) {
-        set_cuda_error(e);
-        return TPN_ERR_CUDA;
-    }
+    // the fold rewrites lists that other ranks may hold in their caches, and this rank's cache is of the old lists
+    rc = shard_new_generation(&s->shard, stream);
+    if (rc != TPN_OK) return rc;
     const StreamView v = make_stream_shard_view(s);
     if (s->shard.world == 1)
         return stream_push_impl<false>(&s->local, v, src_dev, dst_dev, eid_dev, t_dev, batch, ws, stream);

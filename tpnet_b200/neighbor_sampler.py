@@ -22,6 +22,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from .peer import PeerShardMember, rows_on_rank
 
 ArrayOrTensor = Union[np.ndarray, torch.Tensor]
 
@@ -291,7 +292,7 @@ class StreamingRecentSampler:
                          'not answerable from the streaming state (a zero row was returned)')
 
 
-class ShardedStreamingSampler(StreamingRecentSampler):
+class ShardedStreamingSampler(StreamingRecentSampler, PeerShardMember):
     """``StreamingRecentSampler`` over the node-sharded layout of ``ShardedRandomProjection``: node ``u``'s lists live
     on rank ``u % world`` at local row ``u // world``, so a rank holds ``ceil(num_nodes / world) + cache_rows`` list
     rows instead of ``num_nodes`` (``tpn_stream_shard_*``, include/tpnet_b200.h).
@@ -312,14 +313,9 @@ class ShardedStreamingSampler(StreamingRecentSampler):
 
     def __init__(self, num_nodes: int, max_neighbors: int, device: Union[str, torch.device], max_batch: int = 200_000,
                  peers=None, group=None, cache_rows: int = 1 << 16, exchange: str = 'auto'):
-        import torch.distributed as dist
         if exchange not in ('auto', 'peer', 'nccl'):
             raise ValueError("exchange must be 'auto', 'peer' or 'nccl'")
-        if peers is not None:
-            self.world, self.rank = int(peers.world), int(peers.rank)
-        else:
-            self.world = dist.get_world_size(group) if dist.is_initialized() else 1
-            self.rank = dist.get_rank(group) if dist.is_initialized() else 0
+        self._join(num_nodes, peers, group)
         if self.world > 1 and exchange == 'nccl':
             raise NotImplementedError("ShardedStreamingSampler with world > 1 needs exchange='peer' "
                                       "(the sampler pulls remote lists out of peer memory; it has no 'nccl' data plane)")
@@ -327,35 +323,25 @@ class ShardedStreamingSampler(StreamingRecentSampler):
             raise ValueError('a sharded sampler routes node ids through int32 mark tables: num_nodes must be < 2**31')
         if cache_rows < 0:
             raise ValueError('cache_rows must be >= 0')
-        self.group = group
-        self._peers = peers
         self.cache_rows = int(cache_rows) if self.world > 1 else 0
-        self.n_local = (num_nodes - self.rank + self.world - 1) // self.world if num_nodes > self.rank else 0
-        self._connected = False
-        self._dirty = True               # a rank may have folded since the last barrier: barrier before pulling
-        self.barriers = 0                # barriers issued so far (accounting)
-        self._route = {}
         super().__init__(num_nodes, max_neighbors, device, max_batch)
 
     # ------------------------------------------------------------------ set-up
     def _alloc_tables(self) -> None:
         if self.world == 1:
             return super()._alloc_tables()
-        from .peer import PeerBuffer
         dev, C = self.device, self.max_neighbors
         rows = self.n_local + self.cache_rows
         # one peer-visible buffer of the same size on every rank (symmetric memory needs it), the nine tables at the
         # same offsets everywhere: rank q's tables are its base pointer plus these offsets
-        alloc = (self.num_nodes + self.world - 1) // self.world + self.cache_rows
+        alloc = rows_on_rank(self.num_nodes, self.world, 0) + self.cache_rows
         sizes = [alloc * C * 8] * 6 + [alloc * 4, alloc * 4, alloc * 8]
         self._offsets, off = [], 0
         for b in sizes:
             self._offsets.append(off)
             off += (b + 255) // 256 * 256
-        symmetric = self._peers is None or getattr(self._peers, 'symmetric', False)
-        self._lists_buf = PeerBuffer(off, dev, symmetric=symmetric)
-        self._flags_buf = PeerBuffer(4 * max(self.world, 16), dev, symmetric=symmetric)
-        raw = self._lists_buf.tensor((self._lists_buf.nbytes,), torch.uint8)
+        buf = self._peer_buffer('sampler_lists', off, dev)
+        raw = buf.tensor((buf.nbytes,), torch.uint8)
 
         def view(i, dtype, shape):
             n = 1
@@ -370,69 +356,24 @@ class ShardedStreamingSampler(StreamingRecentSampler):
         self._all_cnt = view(6, i32, (rows,))
         self._old_cnt = view(7, i32, (rows,))
         self._newest = view(8, f64, (rows,))
-        self._mark = torch.zeros(self.num_nodes, dtype=i32, device=dev)
-        self._counters = torch.zeros(_lib.SHARD_COUNTERS, dtype=i32, device=dev)
-        self._need = torch.zeros(max(self.cache_rows, 1), dtype=i64, device=dev)
-        self._seq = torch.zeros(1, dtype=i32, device=dev)
-        self._peer_tables = None
-        if hasattr(self._peers, 'publish'):        # in-process ranks: every rank publishes before anyone connects
-            self._peers.publish('sampler_lists', self._lists_buf)
-            self._peers.publish('sampler_flags', self._flags_buf)
+        self._cs = _lib.TpnStreamShard()             # its `shard` is the tpn_shard_t of the base class (one struct)
+        self._init_shard(dev, self.num_nodes, self.cache_rows, 'sampler_flags', self._cs.shard)
+
+    @property
+    def _counters(self) -> torch.Tensor:
+        """The routing counters of the shard (``_shard_tensors['counters']``; ``SHARD_CTR_*`` index them)."""
+        return self._shard_tensors['counters']
 
     def _grow(self, max_batch: int) -> None:
         super()._grow(max_batch)
-        if self.world == 1:
-            return
-        cs = _lib.TpnStreamShard()
-        cs.local = self._c
-        sh = cs.shard
-        sh.world, sh.rank, sh.global_nodes = self.world, self.rank, self.num_nodes
-        sh.num_local_rows, sh.ext_rows = self.n_local, self.cache_rows
-        sh.mark, sh.counters, sh.need_nodes = self._mark.data_ptr(), self._counters.data_ptr(), self._need.data_ptr()
-        sh.barrier_seq = self._seq.data_ptr()
-        if self._peer_tables is not None:
-            sh.peer_flags = self._peer_tables['flags'].data_ptr()
-            cs.peer_lists = self._peer_tables['lists'].data_ptr()
-        self._cs = cs
+        if self.world > 1:
+            self._cs.local = self._c
 
-    def connect(self) -> None:
-        """Rendezvous of the peer-visible list tables (collective; the first push or query does it if the caller did
-        not).  With a ``LocalPeerGroup`` every rank must be constructed first."""
-        if self.world == 1 or self._connected:
-            return
-        import torch.distributed as dist
-        from .peer import SymmPeerGroup
-        if self._peers is None:
-            if not dist.is_initialized():
-                raise RuntimeError('a sharded sampler with world > 1 needs torch.distributed or a PeerGroup')
-            self._peers = SymmPeerGroup(self.group)
-        bases = self._peers.exchange('sampler_lists', self._lists_buf)
-        flags = self._peers.exchange('sampler_flags', self._flags_buf)
-        self._peer_tables = {
-            'lists': torch.tensor([b + o for b in bases for o in self._offsets], dtype=torch.int64, device=self.device),
-            'flags': torch.tensor(flags, dtype=torch.int64, device=self.device)}
-        self._cs.shard.peer_flags = self._peer_tables['flags'].data_ptr()
-        self._cs.peer_lists = self._peer_tables['lists'].data_ptr()
-        self._connected = True
-        self._peers.barrier()            # every rank has mapped every buffer before anyone pulls
-
-    def close(self) -> None:
-        """Collective teardown, as ``ShardedRandomProjection.close``: no rank frees its tables while a peer maps them."""
-        if not self._connected:
-            return
-        torch.cuda.synchronize(self.device)
-        self._peers.barrier()
-        if hasattr(self._peers, 'close'):
-            self._peers.close()
-        self._peers.barrier()
-        self._connected = False
-
-    def _barrier(self) -> None:
-        self.connect()
-        self.barriers += 1
-        if getattr(self._peers, 'host_barriers', False):
-            return          # LocalPeerGroup: the driver of the in-process ranks orders the phases itself (peer.py)
-        _lib.check(_lib.load().tpn_peer_barrier(ctypes.byref(self._cs.shard), self._stream()), 'tpn_peer_barrier')
+    def _connect_tables(self, bases):
+        lists = torch.tensor([b + o for b in bases['sampler_lists'] for o in self._offsets], dtype=torch.int64,
+                             device=self.device)
+        self._cs.peer_lists = lists.data_ptr()
+        return {'lists': lists}
 
     # ------------------------------------------------------------------ API
     def reset(self) -> None:
@@ -455,21 +396,6 @@ class ShardedStreamingSampler(StreamingRecentSampler):
             _lib.check(rc, 'tpn_stream_shard_push')
         self._dirty = True
 
-    def row_split(self, m: int) -> Tuple[int, int, int]:
-        """(per, lo, hi): this rank answers rows [lo, hi) of a call with m rows (ShardedRandomProjection._row_split)."""
-        per = -(-m // self.world)
-        lo = min(self.rank * per, m)
-        return per, lo, min(lo + per, m)
-
-    def _positions(self, lo: int, hi: int) -> torch.Tensor:
-        key = ('positions', lo, hi)
-        t = self._route.get(key)
-        if t is None:
-            if len(self._route) > 8:
-                self._route.clear()
-            t = self._route[key] = torch.arange(lo, hi, dtype=torch.int64, device=self.device)
-        return t
-
     def get_historical_neighbors(self, node_ids: ArrayOrTensor, node_interact_times: ArrayOrTensor,
                                  num_neighbors: int = 20, as_tensors: bool = False):
         """This rank's slice of ``StreamingRecentSampler.get_historical_neighbors`` over the replicated call:
@@ -477,7 +403,7 @@ class ShardedStreamingSampler(StreamingRecentSampler):
         Host ids of the whole call are checked on every rank before anything is launched."""
         m = self._check_query(node_ids, node_interact_times, num_neighbors)
         per, lo, hi = self.row_split(m)
-        keep = self._positions(lo, hi)
+        keep = self._positions(lo, hi, self.device)
         if self.world == 1:
             res = super().get_historical_neighbors(node_ids, node_interact_times, num_neighbors, as_tensors)
             return (keep if as_tensors else keep.cpu().numpy(),) + tuple(res)
@@ -489,16 +415,13 @@ class ShardedStreamingSampler(StreamingRecentSampler):
         out_n = torch.empty(n, K, dtype=torch.int64, device=dev)
         out_e = torch.empty(n, K, dtype=torch.int64, device=dev)
         out_t = torch.empty(n, K, dtype=torch.float64, device=dev)
-        self.connect()
         stream = self._stream()
         # route even an empty slice: the pull that follows then fetches nothing, and every rank takes the barrier
-        rc = lib.tpn_route_nodes(ctypes.byref(self._cs.shard), qn.data_ptr() if n else None, n,
-                                 rows.data_ptr() if n else None, stream)
+        rc = lib.tpn_route_nodes(self._c_shard(), qn.data_ptr() if n else None, n, rows.data_ptr() if n else None,
+                                 stream)
         if rc:
             _lib.check(rc, 'tpn_route_nodes')
-        if self._dirty:
-            self._barrier()              # every rank's fold is done before anyone reads its lists
-            self._dirty = False
+        self._before_pull()              # every rank's fold is done before anyone reads its lists
         _lib.check(lib.tpn_stream_shard_pull(ctypes.byref(self._cs), stream), 'tpn_stream_shard_pull')
         if n:
             rc = lib.tpn_stream_shard_query(ctypes.byref(self._cs), qn.data_ptr(), rows.data_ptr(), qt.data_ptr(), n, K,
@@ -514,20 +437,14 @@ class ShardedStreamingSampler(StreamingRecentSampler):
     def check_errors(self) -> None:
         """``StreamingRecentSampler.check_errors``, then the routing flags: IndexError for an id outside the graph,
         RuntimeError when one generation's remote lists do not fit ``cache_rows``."""
-        code = 0
-        if self.world > 1:
-            code = int(self._counters[_lib.SHARD_CTR_ERROR].item())
-            if code:
-                self._counters[_lib.SHARD_CTR_ERROR] = 0          # cleared with the sampler's flag, by one call
+        err = self._take_shard_error(               # cleared with the sampler's flag, by one call
+            f'node id out of range for a sampler over {self.num_nodes} nodes (routing)',
+            f'the remote lists one batch queries do not fit cache_rows={self.cache_rows}: construct '
+            f'ShardedStreamingSampler with a larger cache_rows',
+            'a peer rank never reached a barrier of the sharded sampler')
         super().check_errors()
-        if code == 0:
-            return
-        if code == 1:
-            raise IndexError(f'node id out of range for a sampler over {self.num_nodes} nodes (routing)')
-        if code == 2:
-            raise RuntimeError(f'the remote lists one batch queries do not fit cache_rows={self.cache_rows}: '
-                               f'construct ShardedStreamingSampler with a larger cache_rows')
-        raise RuntimeError('a peer rank never reached a barrier of the sharded sampler')
+        if err is not None:
+            raise err
 
 
 def get_neighbor_sampler(data, sample_neighbor_strategy: str = 'recent', device: Union[str, torch.device] = 'cuda:0',

@@ -20,13 +20,16 @@ stamps and barrier words must be mapped into every other rank's address space:
                           pointers are simply the other ranks' pointers.  This is how the single-GPU test box
                           runs the complete routed data plane (routing, pulls, barriers, device-side counts);
                           only the NVLink transport itself needs more than one GPU.
+
+``PeerShardMember`` is the rank-local side of that protocol, shared by the sharded state and the sharded sampler.
 """
 from __future__ import annotations
 
 import ctypes
-from typing import Dict, List, Optional
+from typing import Dict, List, Optional, Tuple
 
 import torch
+import torch.distributed as dist
 
 from . import _lib
 
@@ -142,7 +145,6 @@ class SymmPeerGroup(PeerGroup):
     symmetric = True
 
     def __init__(self, group=None):
-        import torch.distributed as dist
         self._dist = dist
         self.group = group if group is not None else dist.group.WORLD
         self.world = dist.get_world_size(self.group)
@@ -172,7 +174,6 @@ class IpcPeerGroup(PeerGroup):
     for why this is not the default)."""
 
     def __init__(self, group=None):
-        import torch.distributed as dist
         self._dist = dist
         self.group = group
         self.world = dist.get_world_size(group)
@@ -206,3 +207,156 @@ class IpcPeerGroup(PeerGroup):
         for p in self._opened:
             self._lib.tpn_ipc_close(p)
         self._opened = []
+
+
+def rows_on_rank(node_num: int, world: int, rank: int) -> int:
+    """Number of global ids u < node_num with u % world == rank (node u lives on rank u % world, row u // world)."""
+    return (node_num - rank + world - 1) // world if node_num > rank else 0
+
+
+class PeerShardMember:
+    """One rank of a node-sharded module with a peer data plane: the rank-local side of the "Barrier protocol" of
+    include/tpnet_b200.h, shared by ``ShardedRandomProjection`` and ``ShardedStreamingSampler``.
+
+    The owner calls ``_join`` first (world, rank, ``n_local``), allocates its peer-visible memory with
+    ``_peer_buffer`` and ``_init_shard`` (the flags buffer and the routing shard: mark table, counters, need list and
+    barrier sequence in ``_shard_tensors``, described by the ``tpn_shard_t`` ``_shard``), and turns the exchanged base
+    pointers into its own tables in ``_connect_tables``.  A module without a peer data plane (world 1, or the 'nccl'
+    plane of the state) calls ``_join`` only: ``_shard`` stays None and nothing peer-visible is allocated."""
+
+    def _join(self, node_num: int, peers: Optional[PeerGroup], group) -> None:
+        """World and rank from ``peers``, else from torch.distributed (world 1 without it); the rows this rank owns."""
+        if peers is not None:
+            self.world, self.rank = int(peers.world), int(peers.rank)
+        else:
+            self.world = dist.get_world_size(group) if dist.is_initialized() else 1
+            self.rank = dist.get_rank(group) if dist.is_initialized() else 0
+        self.group = group
+        self._peers = peers
+        self.n_local = rows_on_rank(node_num, self.world, self.rank)
+        self._peer_bufs: Dict[str, PeerBuffer] = {}
+        self._shard: Optional[_lib.TpnShard] = None
+        self._shard_tensors = {}
+        self._connected = False
+        self._route = {}                 # cached device buffers, keyed by (kind, ...)
+        self._dirty = True               # a rank may have written since the last barrier: barrier before pulling
+        self.barriers = 0                # barriers issued so far (bench accounting)
+
+    def _peer_buffer(self, name: str, nbytes: int, device) -> PeerBuffer:
+        """Zero-filled peer-visible buffer ``name``.  ``nbytes`` must be the same on every rank (symmetric memory
+        needs it).  In-process ranks publish it at once, so every rank constructed can connect."""
+        symmetric = self._peers is None or getattr(self._peers, 'symmetric', False)
+        buf = self._peer_bufs[name] = PeerBuffer(nbytes, device, symmetric=symmetric)
+        if isinstance(self._peers, LocalPeerGroup):
+            self._peers.publish(name, buf)
+        return buf
+
+    def _init_shard(self, device, global_nodes: int, ext_rows: int, flags: str,
+                    shard: Optional[_lib.TpnShard] = None) -> None:
+        """The flags buffer ``flags`` (one barrier word per rank) and the routing shard over ``global_nodes`` ids with
+        ``ext_rows`` cache rows, described in ``shard`` (a new ``TpnShard`` unless the owner embeds one)."""
+        self._flags_name = flags
+        self._peer_buffer(flags, 4 * max(self.world, 16), device)
+        t = self._shard_tensors
+        t['mark'] = torch.zeros(global_nodes, dtype=torch.int32, device=device)
+        t['counters'] = torch.zeros(_lib.SHARD_COUNTERS, dtype=torch.int32, device=device)
+        t['need'] = torch.zeros(max(ext_rows, 1), dtype=torch.int64, device=device)
+        t['seq'] = torch.zeros(1, dtype=torch.int32, device=device)
+        sh = shard if shard is not None else _lib.TpnShard()
+        sh.world, sh.rank, sh.global_nodes = self.world, self.rank, global_nodes
+        sh.num_local_rows, sh.ext_rows = self.n_local, ext_rows
+        sh.mark, sh.counters = t['mark'].data_ptr(), t['counters'].data_ptr()
+        sh.need_nodes, sh.barrier_seq = t['need'].data_ptr(), t['seq'].data_ptr()
+        self._shard = sh
+
+    def _connect_tables(self, bases: Dict[str, List[int]]) -> Dict[str, torch.Tensor]:
+        """The owner's device tables built from every rank's base pointer of each of its buffers (flags excluded),
+        written into its C structs; returned to be kept alive in ``_shard_tensors['tables']``."""
+        raise NotImplementedError
+
+    def connect(self) -> None:
+        """Rendezvous of the peer-visible buffers (collective over the ranks; the first call that needs the peers does
+        it if the caller did not).  With a ``LocalPeerGroup`` every rank must be constructed first."""
+        if self._shard is None or self._connected:
+            return
+        if self._peers is None:
+            if not dist.is_initialized():
+                raise RuntimeError(f'{type(self).__name__} with world > 1 needs torch.distributed or a PeerGroup')
+            self._peers = SymmPeerGroup(self.group)
+        bases = {name: self._peers.exchange(name, buf) for name, buf in self._peer_bufs.items()}
+        flags = torch.tensor(bases.pop(self._flags_name), dtype=torch.int64, device=self._shard_tensors['mark'].device)
+        tables = dict(self._connect_tables(bases), flags=flags)
+        self._shard.peer_flags = flags.data_ptr()
+        self._shard_tensors['tables'] = tables
+        self._connected = True
+        self._peers.barrier()            # every rank has mapped every buffer before anyone launches a pull
+
+    def close(self) -> None:
+        """Collective teardown of the peer data plane: every rank stops using its peers' memory, unmaps it, and only
+        then may anyone free its buffers (freeing an exported allocation that a peer still maps is undefined).  Call
+        it on every rank before dropping the module when another sharded module will be created in the same job."""
+        if not self._connected:
+            return
+        torch.cuda.synchronize(self._shard_tensors['mark'].device)
+        self._peers.barrier()
+        if hasattr(self._peers, 'close'):
+            self._peers.close()
+        self._peers.barrier()
+        self._connected = False
+        del self._shard_tensors['tables']
+
+    def __del__(self):
+        try:                                       # best effort without the barriers (interpreter shutdown, errors)
+            if getattr(self, '_connected', False) and hasattr(self._peers, 'close'):
+                self._peers.close()
+        except Exception:
+            pass
+
+    def _c_shard(self):
+        """byref of the ``tpn_shard_t``, connected."""
+        if not self._connected:
+            self.connect()
+        return ctypes.byref(self._shard)
+
+    def _barrier(self) -> None:
+        self.barriers += 1
+        if getattr(self._peers, 'host_barriers', False):
+            return          # LocalPeerGroup: the driver of the in-process ranks orders the phases itself
+        _lib.check(_lib.load().tpn_peer_barrier(self._c_shard(), self._stream()), 'tpn_peer_barrier')
+
+    def _before_pull(self) -> None:
+        """Peers' writes are ordered before this rank's reads of their rows: one barrier after any write."""
+        if self._dirty:
+            self._barrier()
+            self._dirty = False
+
+    def _take_shard_error(self, out_of_range: str, cache_full: str, no_barrier: str) -> Optional[Exception]:
+        """Reads and clears the sticky routing error ``counters[SHARD_CTR_ERROR]``; the exception it stands for, with
+        the owner's text: IndexError for an id outside the graph (1), RuntimeError when one generation's remote rows do
+        not fit the cache (2) or a peer never reached a barrier (3)."""
+        if self._shard is None:
+            return None
+        ctr = self._shard_tensors['counters']
+        code = int(ctr[_lib.SHARD_CTR_ERROR].item())
+        if code == 0:
+            return None
+        ctr[_lib.SHARD_CTR_ERROR] = 0
+        if code == 1:
+            return IndexError(out_of_range)
+        return RuntimeError(cache_full if code == 2 else no_barrier)
+
+    def row_split(self, m: int) -> Tuple[int, int, int]:
+        """(per, lo, hi): this rank computes rows [lo, hi) of a call with m rows, per = ceil(m / world)."""
+        per = -(-m // self.world)
+        lo = min(self.rank * per, m)
+        return per, lo, min(lo + per, m)
+
+    def _positions(self, lo: int, hi: int, device) -> torch.Tensor:
+        """Device int64 [lo, hi) (cached: the same split recurs every batch)."""
+        key = ('positions', lo, hi)
+        t = self._route.get(key)
+        if t is None:
+            if len(self._route) > 8:
+                self._route.clear()
+            t = self._route[key] = torch.arange(lo, hi, dtype=torch.int64, device=device)
+        return t

@@ -36,7 +36,7 @@ import torch
 import torch.distributed as dist
 
 from . import _lib
-from .peer import IpcPeerGroup, LocalPeerGroup, PeerBuffer, PeerGroup, SymmPeerGroup
+from .peer import IpcPeerGroup, PeerGroup, PeerShardMember, SymmPeerGroup, rows_on_rank
 from .random_projection import _DEFAULT_LOG_EPOCHS, RandomProjectionModule, _round_up
 
 
@@ -46,11 +46,6 @@ def owner_of(ids: np.ndarray, world: int) -> np.ndarray:
 
 def local_row(ids: np.ndarray, world: int) -> np.ndarray:
     return ids // world
-
-
-def rows_on_rank(node_num: int, world: int, rank: int) -> int:
-    """Number of global ids u < node_num with u % world == rank."""
-    return (node_num - rank + world - 1) // world if node_num > rank else 0
 
 
 @dataclass
@@ -178,7 +173,7 @@ class RoutedPairs:
         return self.keep[:m], self.feat[:m]
 
 
-class ShardedRandomProjection(RandomProjectionModule):
+class ShardedRandomProjection(RandomProjectionModule, PeerShardMember):
     """Rank-local part of the node-sharded state.  Same constructor as the reference class plus
     the process group; ``node_num`` is the GLOBAL node count.  ``update`` and
     ``pair_wise_gram`` take the replicated global-id batch; ``pair_wise_gram`` returns the
@@ -189,7 +184,7 @@ class ShardedRandomProjection(RandomProjectionModule):
 
     ``exchange``: 'peer' — routing, NVLink pulls and barriers on the device (module docstring; needs the state
     on CUDA); 'nccl' — host plan + one all_to_all_single; 'auto' — 'peer' when the state is created on a CUDA
-    device (``state_device``), else 'nccl'.  ``peers``: a ``PeerGroup`` (default: ``IpcPeerGroup`` over
+    device (``state_device``), else 'nccl'.  ``peers``: a ``PeerGroup`` (default: ``SymmPeerGroup`` over
     ``group`` when torch.distributed is initialised; ``LocalPeerGroup`` views put several ranks in one
     process).  ``route_cap_factor`` bounds the share of a call's items one rank may own (the launches of the
     rank-local kernels are sized for ``min(1, factor / world)`` of the call; an overflow is flagged, never silent).
@@ -213,12 +208,7 @@ class ShardedRandomProjection(RandomProjectionModule):
             raise ValueError("p0_seed selects the counter-based P_0: leave p0 at its default")
         if exchange not in ('auto', 'peer', 'nccl'):
             raise ValueError("exchange must be 'auto', 'peer' or 'nccl'")
-        self.group = group
-        if peers is not None:
-            self.world, self.rank = int(peers.world), int(peers.rank)
-        else:
-            self.world = dist.get_world_size(group) if dist.is_initialized() else 1
-            self.rank = dist.get_rank(group) if dist.is_initialized() else 0
+        self._join(int(node_num), peers, group)
         sdev = torch.device(state_device) if state_device is not None else None
         if exchange == 'auto':
             exchange = 'peer' if (sdev is not None and sdev.type == 'cuda' and self.world > 1) else 'nccl'
@@ -227,7 +217,6 @@ class ShardedRandomProjection(RandomProjectionModule):
         self.exchange = exchange
         self.route_cap_factor = float(route_cap_factor)
         self.global_node_num = int(node_num)
-        self.n_local = rows_on_rank(self.global_node_num, self.world, self.rank)
         self.ext_rows = int(ext_rows)
         # the width rule uses the GLOBAL node count (TPNet.py:30-33)
         dim = enforce_dim if enforce_dim != -1 else min(int(math.log(edge_num * 2)) * dim_factor, node_num)
@@ -241,17 +230,11 @@ class ShardedRandomProjection(RandomProjectionModule):
         else:
             mine = None
         state_buffer = None
-        self._peer_bufs = {}
-        # one process per GPU: symmetric memory (2 MiB pages; the legacy-IPC mapping is TLB-bound, peer.py);
-        # an explicit PeerGroup (in-process ranks, IPC) brings its own kind of buffer
-        self._symmetric = exchange == 'peer' and (peers is None or getattr(peers, 'symmetric', False))
-        self._rows_alloc = rows_on_rank(self.global_node_num, self.world, 0) + self.ext_rows      # same on every rank
+        rows_alloc = rows_on_rank(self.global_node_num, self.world, 0) + self.ext_rows      # same on every rank
         if exchange == 'peer':
-            rows = self.n_local + self.ext_rows
             stride = _round_up(dim, 8)
-            buf = PeerBuffer(self._rows_alloc * (num_layer + 1) * stride * 4, sdev, symmetric=self._symmetric)
-            self._peer_bufs['state'] = buf
-            state_buffer = buf.tensor((rows, num_layer + 1, stride), torch.float32)
+            buf = self._peer_buffer('state', rows_alloc * (num_layer + 1) * stride * 4, sdev)
+            state_buffer = buf.tensor((self.n_local + self.ext_rows, num_layer + 1, stride), torch.float32)
         super().__init__(node_num=self.n_local + self.ext_rows, edge_num=edge_num, dim_factor=dim_factor,
                          num_layer=num_layer, time_decay_weight=time_decay_weight, device=device, use_matrix=False,
                          beginning_time=beginning_time, not_scale=not_scale, enforce_dim=dim, decay_mode=decay_mode,
@@ -264,22 +247,14 @@ class ShardedRandomProjection(RandomProjectionModule):
         self._send_buf: Optional[torch.Tensor] = None
         self._all_keep: Optional[np.ndarray] = None
         self._planner: Optional[NativePlanner] = None
-        # ---- peer data plane
-        self._peers = peers
-        self._shard: Optional[_lib.TpnShard] = None
-        self._shard_tensors = {}
-        self._route = {}                 # cached routing buffers, keyed by (kind, items)
-        self._dirty = True               # a rank may have written since the last barrier: barrier before pulling
-        self.barriers = 0                # barriers issued so far (bench accounting)
         if exchange == 'peer':
             if self.lazy:
                 # stamps live in peer memory too (a puller copies them with the rows); -1 = never written
-                sb = PeerBuffer(self._rows_alloc * self.num_layer * 4, sdev, symmetric=self._symmetric)
-                self._peer_bufs['stamps'] = sb
+                sb = self._peer_buffer('stamps', rows_alloc * self.num_layer * 4, sdev)
                 self._stamps = sb.tensor((self.node_num, self.num_layer), torch.int32)
                 self._stamps.fill_(-1)
                 self._decay_log = torch.ones(_DEFAULT_LOG_EPOCHS, self.num_layer, dtype=torch.float64, device=sdev)
-            self._peer_bufs['flags'] = PeerBuffer(4 * max(self.world, 16), sdev, symmetric=self._symmetric)
+            self._init_shard(sdev, self.global_node_num, self.ext_rows, 'flags')
 
     # ------------------------------------------------------------------ helpers
     def init_p0_on_device(self, seed: int) -> None:
@@ -344,69 +319,13 @@ class ShardedRandomProjection(RandomProjectionModule):
             self._stamps[self.n_local:self.n_local + R].fill_(self._h.epoch)     # received rows are current
         self.exchanged_rows += R
 
-    # ------------------------------------------------------------------ peer data plane: set-up
-    def connect(self) -> None:
-        """Rendezvous of the peer-visible buffers (collective over the ranks of the group; the first routed call
-        does it if the caller did not).  With a ``LocalPeerGroup`` every rank must be constructed first."""
-        if self.exchange != 'peer' or self._shard is not None:
-            return
+    # ------------------------------------------------------------------ peer data plane
+    def _connect_tables(self, bases):
         dev = self._require_cuda()
-        if self._peers is None:
-            if not dist.is_initialized():
-                raise RuntimeError("exchange='peer' with world > 1 needs torch.distributed or a PeerGroup")
-            self._peers = SymmPeerGroup(self.group)
-        tables = {}
-        for name in ('state', 'stamps', 'flags'):
-            if name in self._peer_bufs:
-                ptrs = self._peers.exchange(name, self._peer_bufs[name])
-                tables[name] = torch.tensor(ptrs, dtype=torch.int64, device=dev)
-        t = self._shard_tensors
-        t['tables'] = tables
-        t['mark'] = torch.zeros(self.global_node_num, dtype=torch.int32, device=dev)
-        t['counters'] = torch.zeros(_lib.SHARD_COUNTERS, dtype=torch.int32, device=dev)
-        t['need'] = torch.zeros(max(self.ext_rows, 1), dtype=torch.int64, device=dev)
-        t['seq'] = torch.zeros(1, dtype=torch.int32, device=dev)
-        sh = _lib.TpnShard()
-        sh.world, sh.rank = self.world, self.rank
-        sh.global_nodes = self.global_node_num
-        sh.num_local_rows = self.n_local
-        sh.ext_rows = self.ext_rows
-        sh.peer_data = tables['state'].data_ptr()
-        sh.peer_stamps = tables['stamps'].data_ptr() if 'stamps' in tables else None
-        sh.peer_flags = tables['flags'].data_ptr()
-        sh.mark = t['mark'].data_ptr()
-        sh.counters = t['counters'].data_ptr()
-        sh.need_nodes = t['need'].data_ptr()
-        sh.barrier_seq = t['seq'].data_ptr()
-        self._shard = sh
-        self._peers.barrier()            # every rank has mapped every buffer before anyone launches a pull
-
-    def close(self) -> None:
-        """Collective teardown of the peer data plane: every rank stops using its peers' memory, unmaps it, and only
-        then may anyone free its buffers (freeing an exported allocation that a peer still maps is undefined).  Call
-        it on every rank before dropping the module when another sharded module will be created in the same job."""
-        if self._shard is None or self._peers is None:
-            return
-        if self._state.is_cuda:
-            torch.cuda.synchronize(self._state.device)
-        self._peers.barrier()
-        if hasattr(self._peers, 'close'):
-            self._peers.close()
-        self._peers.barrier()
-        self._shard = None
-        self._shard_tensors = {}
-
-    def __del__(self):
-        try:                                       # best effort without the barriers (interpreter shutdown, errors)
-            if getattr(self, '_shard', None) is not None and hasattr(self._peers, 'close'):
-                self._peers.close()
-        except Exception:
-            pass
-
-    def _c_shard(self):
-        if self._shard is None:
-            self.connect()
-        return ctypes.byref(self._shard)
+        tables = {name: torch.tensor(ptrs, dtype=torch.int64, device=dev) for name, ptrs in bases.items()}
+        self._shard.peer_data = tables['state'].data_ptr()
+        self._shard.peer_stamps = tables['stamps'].data_ptr() if 'stamps' in tables else None
+        return tables
 
     def _cap(self, items: int) -> int:
         """Launch capacity for the rank-local kernels of a call with `items` work items in total."""
@@ -430,25 +349,18 @@ class ShardedRandomProjection(RandomProjectionModule):
             self._route[key] = buf
         return buf
 
-    def _barrier(self) -> None:
-        self.barriers += 1
-        if getattr(self._peers, 'host_barriers', False):
-            return          # LocalPeerGroup: the driver of the in-process ranks orders the phases itself (peer.py)
-        _lib.check(_lib.load().tpn_peer_barrier(self._c_shard(), self._stream()), 'tpn_peer_barrier')
-
     def _pull(self) -> None:
-        """Peers' writes are ordered before this rank's reads of their rows (one barrier after any write), then the
-        cache slots handed out by the latest routing call are filled from the owners' memory."""
-        if self._dirty:
-            self._barrier()
-            self._dirty = False
+        """The barrier a write calls for, then the cache slots handed out by the latest routing call are filled from the
+        owners' memory."""
+        self._before_pull()
         _lib.check(_lib.load().tpn_pull_rows(self._c_state(), self._c_shard(), self._stream()), 'tpn_pull_rows')
 
     def _state_written(self) -> None:
         """After any write to the local rows: cached copies held by (and of) other ranks are stale."""
         self._dirty = True
-        if self._shard is not None:
-            _lib.check(_lib.load().tpn_shard_new_generation(self._c_shard(), self._stream()), 'tpn_shard_new_generation')
+        if self._shard is not None:                   # local tables only: this does not connect
+            _lib.check(_lib.load().tpn_shard_new_generation(ctypes.byref(self._shard), self._stream()),
+                       'tpn_shard_new_generation')
 
     def _update_peer(self, src_node_ids, dst_node_ids, node_interact_times, next_time) -> None:
         pending = self.update_begin(src_node_ids, dst_node_ids, node_interact_times, next_time)
@@ -792,23 +704,6 @@ class ShardedRandomProjection(RandomProjectionModule):
     # (no device count, no capacity padding, no device -> host read).  The rows a rank reads are routed
     # (tpn_route_nodes: own rows, or cache slots of the current generation) and pulled, then the plain kernels run on
     # the translated rows of the local state.
-    def _row_split(self, m: int) -> Tuple[int, int, int]:
-        """(per, lo, hi): this rank computes rows [lo, hi) of a call with m rows."""
-        per = -(-m // self.world)
-        lo = min(self.rank * per, m)
-        return per, lo, min(lo + per, m)
-
-    def _positions(self, lo: int, hi: int) -> torch.Tensor:
-        """Device int64 [lo, hi) (cached: the same split recurs every batch)."""
-        key = ('positions', lo, hi)
-        t = self._route.get(key)
-        if t is None:
-            t = torch.arange(lo, hi, dtype=torch.int64, device=self._state.device)
-            if len(self._route) > 8:
-                self._route.clear()
-            self._route[key] = t
-        return t
-
     def _check_node_call(self, what: str) -> None:
         if self.world > 1 and self.exchange != 'peer':
             raise NotImplementedError(f"{what} on a sharded state with world > 1 needs exchange='peer' "
@@ -890,13 +785,13 @@ class ShardedRandomProjection(RandomProjectionModule):
         k = int(neighbor_node_ids.shape[1])
         if len(src_node_ids) != m or len(dst_node_ids) != m:
             raise ValueError('src and dst id arrays must have one entry per row of neighbor_node_ids')
-        per, lo, hi = self._row_split(m)
+        per, lo, hi = self.row_split(m)
         n = hi - lo
         if sliced_neighbors and int(neighbor_node_ids.shape[0]) != n:
             raise ValueError(f'sliced_neighbors: this rank computes rows [{lo}, {hi}) of {m}, so neighbor_node_ids must '
                              f'have {n} rows (it has {int(neighbor_node_ids.shape[0])})')
         nbr = neighbor_node_ids if sliced_neighbors else neighbor_node_ids[lo:hi]
-        keep = self._positions(lo, hi)
+        keep = self._positions(lo, hi, dev)
         resident = all(isinstance(a, torch.Tensor) and a.is_cuda for a in (neighbor_node_ids, src_node_ids, dst_node_ids))
         if self.world == 1:
             flat = neighbor_node_ids.reshape(-1)
@@ -927,7 +822,7 @@ class ShardedRandomProjection(RandomProjectionModule):
         if not gather:
             return keep, feat
         m = int(len(src_node_ids))
-        return self._gather_slices(feat, self._row_split(m)[0], m)
+        return self._gather_slices(feat, self.row_split(m)[0], m)
 
     def _gather_state_rows(self, ptr: int, n: int) -> torch.Tensor:
         out = torch.empty(self.num_layer + 1, n, self.dim, dtype=torch.float32, device=self._state.device)
@@ -951,13 +846,13 @@ class ShardedRandomProjection(RandomProjectionModule):
             ptr = self._rank_ids_to_device([node_ids], ['id'])[0] if n else 0
             out = self._gather_state_rows(ptr, n)
             return [out[i] for i in range(self.num_layer + 1)]
-        per, lo, hi = self._row_split(n)
+        per, lo, hi = self.row_split(n)
         rows = self._route_node_rows(node_ids[lo:hi])
         out = self._gather_state_rows(rows.data_ptr(), hi - lo)
         if gather:
             full = self._gather_slices(out.transpose(0, 1), per, n).transpose(0, 1).contiguous()
             return [full[i] for i in range(self.num_layer + 1)]
-        return self._positions(lo, hi), [out[i] for i in range(self.num_layer + 1)]
+        return self._positions(lo, hi, dev), [out[i] for i in range(self.num_layer + 1)]
 
     # ------------------------------------------------------------------ state changes invalidate the remote-row caches
     def _before_write(self) -> None:
@@ -990,16 +885,13 @@ class ShardedRandomProjection(RandomProjectionModule):
 
     def check_errors(self) -> None:
         super().check_errors()
-        if self._shard is not None:
-            code = int(self._shard_tensors['counters'][_lib.SHARD_CTR_ERROR].item())
-            if code:
-                self._shard_tensors['counters'][_lib.SHARD_CTR_ERROR] = 0
-                if code == 1:
-                    raise IndexError(f'node id out of range for node_num {self.global_node_num} in a sharded batch')
-                if code == 2:
-                    raise RuntimeError(f'the {self.ext_rows} extension rows cannot hold the remote rows of one '
-                                       f'generation: construct ShardedRandomProjection with a larger ext_rows')
-                raise RuntimeError('a peer rank never reached a barrier of the sharded data plane')
+        err = self._take_shard_error(
+            f'node id out of range for node_num {self.global_node_num} in a sharded batch',
+            f'the {self.ext_rows} extension rows cannot hold the remote rows of one generation: construct '
+            f'ShardedRandomProjection with a larger ext_rows',
+            'a peer rank never reached a barrier of the sharded data plane')
+        if err is not None:
+            raise err
 
     def gather_global(self) -> List[torch.Tensor]:
         """All-gathers the L+1 global [N, d] matrices (tests / small graphs only)."""
