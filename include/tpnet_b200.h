@@ -59,7 +59,7 @@
 extern "C" {
 #endif
 
-#define TPN_ABI_VERSION 15
+#define TPN_ABI_VERSION 16
 
 #define TPN_MAX_LAYERS 4
 
@@ -552,6 +552,71 @@ int tpn_stream_shard_pull(const tpn_stream_shard_t* s, void* stream);
 int tpn_stream_shard_query(const tpn_stream_shard_t* s, const int64_t* q_nodes_dev, const int64_t* q_rows_dev,
                            const double* q_times_dev, int64_t n, int num_neighbors, int64_t* out_nbr_dev,
                            int64_t* out_eid_dev, double* out_times_dev, void* stream);
+
+/*
+ * ---------------------------------------------------------------------------------------------------------
+ * Negative edge sampler on the device: DyGLib's NegativeEdgeSampler (the reference's utils/utils.py:315-505) with
+ * its three strategies, drawn from a counter-based generator instead of numpy's MT19937 — the same sets, sizes and
+ * ordering rule, not the same draws.  S, D = sorted unique src / dst ids; W(a, b) = the distinct (src, dst) of the
+ * edges with a <= t <= b; f(key) = the first time of an edge.
+ * Tables (tpn_neg_sampler_build; node ids < 2^id_bits <= 2^32, edge keys are two uint32 words):
+ *   T : the edges stably sorted by time (t_src, t_dst, t_time) and, per edge, t_fpos = the F position of its key;
+ *       a window [s, e] is the range [#{t < s}, #{t <= e}) of T.
+ *   F : the distinct keys sorted by (f, src, dst) (f_src, f_dst, f_time): W(min t, s) is the prefix F[0, #{f <= s}).
+ *   S, D.
+ * A call (tpn_neg_sampler_sample, s = start, e = end, c = call index, key = (seed, c)):
+ *   random     : out[i] = (S[hi64(x0 * |S|)], D[hi64(x1 * |D|)]), x = Philox4x64-10((i, 0, 4, 0), key).
+ *   historical : domain F[0, h), h = #{f <= s};  inductive: F[o, max(o, h)), o = #{f <= last_observed_time}.
+ *                Hc = domain minus W(s, e);  k = min(size, |Hc|): the first k elements of a keyed permutation of the
+ *                domain (tag 1) that are not in W(s, e), in permutation order.
+ *                If size > |Hc|: first the fill, then all of Hc.  Fill = size - |Hc| elements of
+ *                U = S x D minus the batch's pairs, pair index q = i_S * |D| + i_D: the first of a permutation of
+ *                [0, |S||D|) (tag 2) outside the batch; when |U| < fill: out[j] = U[hi64(x0 * |U|)] over U in index
+ *                order, x = Philox((j, 0, 3, 0), key).  |U| == 0 sets TPN_NEG_ERR_EMPTY (the reference asserts) and
+ *                writes -1.
+ *   Permutation of [0, n): a balanced 4-round Feistel network on m bits (m the smallest even number >= 2 with
+ *   2^m >= n), round r: (L, R) -> (R, L ^ (Philox((R, r, tag, 0), key).x0 mod 2^(m/2))), cycle-walking until < n.
+ * Everything is integer arithmetic and exact f64 comparisons: the output depends only on (seed, c, inputs), not on
+ * the grid or the device.  Every call is asynchronous, allocation-free and, with start_dev / end_dev, capturable.
+ */
+#define TPN_NEG_RANDOM 0
+#define TPN_NEG_HISTORICAL 1
+#define TPN_NEG_INDUCTIVE 2
+#define TPN_NEG_ERR_EMPTY 1            /* a fill found S x D entirely inside the batch                             */
+#define TPN_NEG_COUNTS 4               /* counts: [0] distinct keys, [1] |S|, [2] |D|, [3] TPN_NEG_ERR_* bits (sticky) */
+typedef struct tpn_neg_sampler {
+    int64_t   num_edges;               /* E, 1 .. 2^31 - 2^12                                                     */
+    int32_t   id_bits;                 /* every node id < 2^id_bits, 1..32 (sets the radix passes)               */
+    int32_t   timed;                   /* 1: T, F and mark are built (historical / inductive); 0: S and D only   */
+    uint64_t  seed;
+    double    last_observed_time;      /* inductive: observed = the keys with f <= this                          */
+    uint32_t* t_src;                   /* device [E]                                                              */
+    uint32_t* t_dst;                   /* device [E]                                                              */
+    double*   t_time;                  /* device [E]                                                              */
+    uint32_t* t_fpos;                  /* device [E]                                                              */
+    uint32_t* f_src;                   /* device [E] (the first counts[0] are used)                               */
+    uint32_t* f_dst;                   /* device [E]                                                              */
+    double*   f_time;                  /* device [E]                                                              */
+    uint32_t* mark;                    /* device [E], zero between calls                                          */
+    uint32_t* uniq_src;                /* device [min(E, 2^id_bits)]: S                                           */
+    uint32_t* uniq_dst;                /* device [min(E, 2^id_bits)]: D                                           */
+    int32_t*  counts;                  /* device int32[TPN_NEG_COUNTS]                                            */
+} tpn_neg_sampler_t;
+
+/* Scratch bytes of a build of num_edges edges (0: none) and of a call of `size` negatives with a batch of `batch`
+ * edges (0: none); the larger of the two. */
+size_t tpn_neg_sampler_workspace_bytes(int64_t num_edges, int64_t size, int64_t batch);
+/* Builds S, D and (timed) T and F from src_dev / dst_dev int64[E] and t_dev float64[E] (not sorted; t_dev may be
+ * NULL when !timed), zeroes mark and the error bits.  Ids must lie in [0, 2^id_bits) and times must not be NaN (the
+ * caller checks both). */
+int tpn_neg_sampler_build(const tpn_neg_sampler_t* s, const int64_t* src_dev, const int64_t* dst_dev,
+                          const double* t_dev, void* ws_dev, size_t ws_bytes, void* stream);
+/* One `sample` call: out_src_dev / out_dst_dev int64[size].  batch_src_dev / batch_dst_dev int64[batch] (any ids; ids
+ * outside S or D exclude nothing).  start_dev / end_dev: NULL (use start / end) or device doubles read by the kernels. */
+int tpn_neg_sampler_sample(const tpn_neg_sampler_t* s, int strategy, uint64_t call, int64_t size,
+                           const int64_t* batch_src_dev, const int64_t* batch_dst_dev, int64_t batch, double start,
+                           double end, const double* start_dev, const double* end_dev, int64_t* out_src_dev,
+                           int64_t* out_dst_dev, void* ws_dev, size_t ws_bytes, void* stream);
 
 #ifdef __cplusplus
 }

@@ -107,7 +107,7 @@ def diff(a, b):
 
 def parity_run(shape_name: str, epochs: int, gpu: int = 0, edges: int = 0, src: int = 0, dst: int = 0,
                negative: str = 'random', log_dir: str = os.path.join(ROOT, 'gpurun_out', 'apauc'), timeout: int = 3000,
-               train_both: bool = True):
+               train_both: bool = True, gpu_neg_arm: bool = False):
     if not os.path.isfile(os.path.join(REF, 'models', 'TPNet.py')):
         raise FileNotFoundError('oracle/_ref/TPNet missing: run `python oracle/make_ref.py` where /root/reference exists')
     dataset = make_dataset(shape_name, edges, src, dst)
@@ -142,6 +142,17 @@ def parity_run(shape_name: str, epochs: int, gpu: int = 0, edges: int = 0, src: 
     res['eval_max_abs_diff'] = diff(res['eval_stock'], res['eval_dropin'])
     res['tolerance'] = 0.001
     res['pass_eval'] = res['eval_max_abs_diff'] <= 0.001
+    if gpu_neg_arm:
+        # the same checkpoint with the GPU neighbour sampler, without and then with the GPU negative sampler; the
+        # negative sampler draws other negatives from the same sets, so this arm is compared, not held to parity
+        for prefix, flags in (('xevalnbr', ['--tpn-gpu-sampler']),
+                              ('xevalneg', ['--tpn-gpu-sampler', '--tpn-gpu-neg-sampler'])):
+            shutil.copyfile(os.path.join(models, f'stock_link_{dataset}_TPNet_seed0.pkl'),
+                            os.path.join(models, f'{prefix}_link_{dataset}_TPNet_seed0.pkl'))
+            res['seconds'][f'eval_{prefix}'] = run_script('evaluate_link_prediction.py', prefix, dataset, shape_name,
+                                                          False, gpu, ev + flags, log_dir, timeout)
+            res[f'eval_{prefix}'] = read_metrics(os.path.join(results, f'{prefix}_link_{negative}_{dataset}_TPNet_seed0.json'))
+        res['eval_neg_sampler_max_abs_diff'] = diff(res['eval_stock'], res['eval_xevalneg'])
     if train_both:
         res['pass_train'] = res['train_max_abs_diff'] <= 0.001
     return res
@@ -157,11 +168,13 @@ def main():
     ap.add_argument('--gpu', type=int, default=0)
     ap.add_argument('--negative', default='random', choices=['random', 'historical', 'inductive'])
     ap.add_argument('--no-train-dropin', action='store_true')
+    ap.add_argument('--gpu-neg-arm', action='store_true',
+                    help='also evaluate the stock checkpoint with --tpn-gpu-sampler, then adding --tpn-gpu-neg-sampler')
     ap.add_argument('--timeout', type=int, default=3000)
     ap.add_argument('--out', default='')
     a = ap.parse_args()
     res = parity_run(a.shape, a.epochs, a.gpu, a.edges, a.src, a.dst, a.negative, timeout=a.timeout,
-                     train_both=not a.no_train_dropin)
+                     train_both=not a.no_train_dropin, gpu_neg_arm=a.gpu_neg_arm)
     line = json.dumps(res, indent=1)
     print(line)
     if a.out:

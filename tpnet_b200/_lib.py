@@ -21,7 +21,7 @@ TPN_ERR_INDEX = -6
 STAGE_RAW, STAGE_ID_WRAP, STAGE_ID = 0, 1, 2
 TPN_MAX_LAYERS = 4
 UPDATE_WHOLE, UPDATE_PREPARE, UPDATE_APPLY = 0, 1, 2
-ABI_VERSION = 15
+ABI_VERSION = 16
 
 #: every symbol include/tpnet_b200.h declares (tests assert the .so exports all of them)
 EXPORTED_SYMBOLS = (
@@ -35,7 +35,8 @@ EXPORTED_SYMBOLS = (
     'tpn_peer_barrier', 'tpn_shard_new_generation', 'tpn_peer_alloc', 'tpn_peer_free', 'tpn_ipc_export', 'tpn_ipc_open',
     'tpn_ipc_close', 'tpn_stream_sampler_workspace_bytes', 'tpn_stream_sampler_reset', 'tpn_stream_sampler_push',
     'tpn_stream_sampler_query', 'tpn_stream_shard_reset', 'tpn_stream_shard_push', 'tpn_stream_shard_pull',
-    'tpn_stream_shard_query', 'tpn_init_projection',
+    'tpn_stream_shard_query', 'tpn_init_projection', 'tpn_neg_sampler_workspace_bytes', 'tpn_neg_sampler_build',
+    'tpn_neg_sampler_sample',
 )
 
 SHARD_CTR_NEED, SHARD_CTR_PREV, SHARD_CTR_ERROR, SHARD_COUNTERS = 0, 1, 2, 8
@@ -117,6 +118,28 @@ class TpnStreamShard(ctypes.Structure):
     ]
 
 
+class TpnNegSampler(ctypes.Structure):
+    """Mirror of ``tpn_neg_sampler_t`` (include/tpnet_b200.h)."""
+    _fields_ = [
+        ('num_edges', c_int64),
+        ('id_bits', c_int32),
+        ('timed', c_int32),
+        ('seed', c_uint64),
+        ('last_observed_time', c_double),
+        ('t_src', c_void_p),
+        ('t_dst', c_void_p),
+        ('t_time', c_void_p),
+        ('t_fpos', c_void_p),
+        ('f_src', c_void_p),
+        ('f_dst', c_void_p),
+        ('f_time', c_void_p),
+        ('mark', c_void_p),
+        ('uniq_src', c_void_p),
+        ('uniq_dst', c_void_p),
+        ('counts', c_void_p),
+    ]
+
+
 class TpnError(RuntimeError):
     def __init__(self, code: int, where: str, detail: str = ''):
         self.code = code
@@ -166,6 +189,15 @@ def _declare(lib: ctypes.CDLL) -> None:
         fn.argtypes = [POINTER(TpnState), c_void_p]
     lib.tpn_init_projection.restype = c_int
     lib.tpn_init_projection.argtypes = [POINTER(TpnState), c_int64, c_int64, c_int64, c_uint64, c_uint64, c_void_p]
+    lib.tpn_neg_sampler_workspace_bytes.restype = c_size_t
+    lib.tpn_neg_sampler_workspace_bytes.argtypes = [c_int64, c_int64, c_int64]
+    lib.tpn_neg_sampler_build.restype = c_int
+    lib.tpn_neg_sampler_build.argtypes = [POINTER(TpnNegSampler), c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
+                                          c_void_p]
+    lib.tpn_neg_sampler_sample.restype = c_int
+    lib.tpn_neg_sampler_sample.argtypes = [POINTER(TpnNegSampler), c_int, c_uint64, c_int64, c_void_p, c_void_p, c_int64,
+                                           c_double, c_double, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                           c_size_t, c_void_p]
     lib.tpn_sampler_recent.restype = c_int
     lib.tpn_sampler_recent.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int64,
                                        c_int, c_void_p, c_void_p, c_void_p, c_void_p]

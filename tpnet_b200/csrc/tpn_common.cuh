@@ -166,6 +166,29 @@ __device__ __forceinline__ void axpy2_rn(float2& acc, const float2& x, float w) 
     acc.y = __fadd_rn(acc.y, p.y);
 }
 
+// ---------------------------------------------------------------- counter-based generator (tpn_p0.cu, tpn_negsampler.cu)
+// Philox4x64-10 (Salmon et al., SC'11; the Random123 constants, the same bijection as numpy's np.random.Philox).
+constexpr unsigned long long kPhiloxM0 = 0xD2E7470EE14C6C93ull;
+constexpr unsigned long long kPhiloxM1 = 0xCA5A826395121157ull;
+constexpr unsigned long long kPhiloxW0 = 0x9E3779B97F4A7C15ull;
+constexpr unsigned long long kPhiloxW1 = 0xBB67AE8584CAA73Bull;
+
+__device__ __forceinline__ void philox4x64_10(unsigned long long x[4], unsigned long long k0, unsigned long long k1) {
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        if (r > 0) {
+            k0 += kPhiloxW0;
+            k1 += kPhiloxW1;
+        }
+        const unsigned long long hi0 = __umul64hi(kPhiloxM0, x[0]), lo0 = kPhiloxM0 * x[0];
+        const unsigned long long hi1 = __umul64hi(kPhiloxM1, x[2]), lo1 = kPhiloxM1 * x[2];
+        x[0] = hi1 ^ x[1] ^ k0;
+        x[1] = lo1;
+        x[2] = hi0 ^ x[3] ^ k1;
+        x[3] = lo0;
+    }
+}
+
 // ---------------------------------------------------------------- mbarrier / bulk-copy (TMA) wrappers
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 

@@ -14,6 +14,9 @@ What it does before handing control to the script (``runpy``, ``__name__ == '__m
   * with ``--tpn-gpu-sampler`` (an option of the launcher, removed before the script sees its arguments):
     ``utils.utils.get_neighbor_sampler`` returns ``tpnet_b200.neighbor_sampler.RecentNeighborSampler`` for
     the `recent` strategy (the one TPNet uses; any other strategy still gets the reference's sampler).
+  * with ``--tpn-gpu-neg-sampler`` (also consumed here): ``utils.utils.NegativeEdgeSampler`` is
+    ``tpnet_b200.NegativeEdgeSampler`` on the script's device, for every strategy.  Same sets, sizes and ordering
+    rule, different draws (a counter-based generator instead of numpy's MT19937): not a parity arm.
   * with ``--tpn-stock`` (also consumed here): NOTHING is swapped — the reference's own class runs, with only the
     Python >= 3.11 ``random.sample`` shim applied.  This is the comparison arm of ``scripts/apauc_parity.py``.
   * ``--gpu G``: ``torch.cuda.set_device(G)`` before the script starts (the scripts only build the string
@@ -65,7 +68,26 @@ def use_gpu_sampler(device: str = 'cuda:0') -> None:
     ref_utils.get_neighbor_sampler = get_neighbor_sampler
 
 
-def install(reference_dir: str, gpu_sampler: bool = False, device: str = 'cuda:0'):
+def use_gpu_neg_sampler(device: str = 'cuda:0') -> None:
+    """``utils.utils.NegativeEdgeSampler`` (utils/utils.py:315-505) -> the GPU negative sampler."""
+    import utils.utils as ref_utils                         # the reference's module, unmodified
+
+    from .negative_sampler import NegativeEdgeSampler
+    if getattr(ref_utils.NegativeEdgeSampler, '_tpn_gpu_neg_sampler', False):
+        return
+
+    class GpuNegativeEdgeSampler(NegativeEdgeSampler):
+        _tpn_gpu_neg_sampler = True
+
+        def __init__(self, src_node_ids, dst_node_ids, interact_times=None, last_observed_time=None,
+                     negative_sample_strategy: str = 'random', seed: int = None):
+            super().__init__(src_node_ids, dst_node_ids, interact_times, last_observed_time,
+                             negative_sample_strategy, seed, device=device)
+
+    ref_utils.NegativeEdgeSampler = GpuNegativeEdgeSampler
+
+
+def install(reference_dir: str, gpu_sampler: bool = False, device: str = 'cuda:0', gpu_neg_sampler: bool = False):
     """Makes the reference importable and swaps in the drop-in class.  Returns ``models.TPNet``."""
     reference_dir = os.path.abspath(reference_dir)
     if not os.path.isfile(os.path.join(reference_dir, 'models', 'TPNet.py')):
@@ -80,6 +102,8 @@ def install(reference_dir: str, gpu_sampler: bool = False, device: str = 'cuda:0
         allow_sampling_from_sets()
     if gpu_sampler:
         use_gpu_sampler(device)
+    if gpu_neg_sampler:
+        use_gpu_neg_sampler(device)
     return ref_tpnet
 
 
@@ -87,7 +111,7 @@ def main(argv: List[str]) -> None:
     if len(argv) < 2:
         raise SystemExit('usage: python -m tpnet_b200.launch <TPNet checkout> <script.py> [script arguments ...]')
     reference_dir, script = os.path.abspath(argv[0]), argv[1]
-    own = ('--tpn-gpu-sampler', '--tpn-stock')
+    own = ('--tpn-gpu-sampler', '--tpn-gpu-neg-sampler', '--tpn-stock')
     rest = [a for a in argv[2:] if a not in own]
     gpu = 0
     if '--gpu' in rest and rest.index('--gpu') + 1 < len(rest):      # the scripts' own device option (load_configs.py)
@@ -103,7 +127,8 @@ def main(argv: List[str]) -> None:
         if sys.version_info >= (3, 11):
             allow_sampling_from_sets()
     else:
-        install(reference_dir, gpu_sampler='--tpn-gpu-sampler' in argv[2:], device=f'cuda:{gpu}')
+        install(reference_dir, gpu_sampler='--tpn-gpu-sampler' in argv[2:], device=f'cuda:{gpu}',
+                gpu_neg_sampler='--tpn-gpu-neg-sampler' in argv[2:])
     os.chdir(reference_dir)
     for d in ('logs', 'saved_models', 'saved_results'):     # the scripts expect these to exist or create them lazily
         os.makedirs(os.path.join(reference_dir, d), exist_ok=True)
